@@ -5,6 +5,7 @@ queries/sec and p50 latency, exact top-10 over 100M x 384 fp16).
     python bench.py [--gpus N] [--steps K] [--warmup W] [--rows R] [--batch B] [--k 10]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...      # the CPU arm (oracle port) on the host cores
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's results as DIR/<name>.npy
 
 A step = one batch of B queries (default 1024: the throughput configuration) answered against the
 whole corpus (R rows, sharded by id range over the N GPUs: strong scaling).
@@ -30,6 +31,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 SEED = 0xDA5EA2C4
 DIM = 384
@@ -60,7 +62,36 @@ def parse():
     ap.add_argument("--parity-rows", type=int, default=2_000_000)
     ap.add_argument("--no-hnsw", action="store_true", help="reference arm: skip the HNSW stand-in (build takes ~1 min)")
     ap.add_argument("--cpu-budget-s", type=float, default=150.0, help="reference arm: wall-clock budget of the exact-scan steps")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the timed path returned in its last step (labels, distances, "
+                         "counts; float64 / float32) as DIR/<name>.npy, so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64_000_000
+NPY_HEADER_BYTES = 1024  # room left per file for the .npy header
+
+
+def dump_outputs(out_dir, labels, distances, counts):
+    """The results of one batch as DIR/{labels,distances,counts}.npy (labels and counts as float64: exact below 2^53).
+    A batch whose results exceed DUMP_LIMIT_BYTES is cut to a fixed, seeded sample of its queries, listed in query_rows.npy."""
+    labels = np.asarray(labels).astype(np.float64)
+    distances = np.asarray(distances).astype(np.float32)
+    counts = np.asarray(counts).astype(np.float64)
+    nq = labels.shape[0]
+    per_query = labels[0].nbytes + distances[0].nbytes + counts[0].nbytes + 8 if nq else 1
+    budget = DUMP_LIMIT_BYTES - 4 * NPY_HEADER_BYTES
+    out = {"labels": labels, "distances": distances, "counts": counts}
+    if nq * per_query > budget:
+        rows = np.sort(np.random.default_rng(SEED).choice(nq, budget // per_query, replace=False))
+        out = {name: a[rows] for name, a in out.items()}
+        out["query_rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def ncu_traffic_ratio(kernel_key: str):
@@ -164,7 +195,7 @@ def cpu_arm(args, steps, warmup, rows_total, budget_s):
     times = []
     for s_ in range(warmup + steps):
         t0 = time.perf_counter()
-        O.cpu_scan_f16(stored, None, qs, args.k, threads=threads)
+        last = O.cpu_scan_f16(stored, None, qs, args.k, threads=threads)
         dt = time.perf_counter() - t0
         if s_ >= warmup:
             times.append(dt)
@@ -177,6 +208,7 @@ def cpu_arm(args, steps, warmup, rows_total, budget_s):
         "ms_per_step": statistics.mean(times) * 1e3,            # what a step really took here (over the sample)
         "ms_per_step_scaled_to_full_corpus": step_s * 1e3,     # what `value` is computed from
         "sample_rows": sample, "scale": scale,
+        "last_step": last[:3],  # (labels, distances, counts) of the last timed step, over the sample
     }
 
 
@@ -263,6 +295,8 @@ def run_reference(args):
     }
     if not args.no_hnsw:
         line["hnsw_stand_in"] = hnsw_arm()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *r["last_step"])
     print_json(line)
 
 
@@ -271,7 +305,7 @@ def run_ours(args):
     import torch.distributed as dist
 
     from dawnsearch_b200 import synth as O  # workload generator (numpy twin of the device generator)
-    from dawnsearch_b200.sharded import ShardedIndex, shard_range
+    from dawnsearch_b200.sharded import ResultBlock, ShardedIndex, shard_range
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -315,7 +349,8 @@ def run_ours(args):
         return float(t.item())
 
     def timed_device(queries_dev, kk, steps, warm, sample_clocks=False):
-        """Device-resident timing: CUDA events on the launching stream + the library's own per-kernel events."""
+        """Device-resident timing: CUDA events on the launching stream + the library's own per-kernel events.
+        Also returns the result block of the last step (a workspace buffer the next search of that shape overwrites)."""
         # back-to-back batches: the exchange of batch i overlaps the search of batch i+1 (not worth it
         # for single queries, where the side-stream bookkeeping costs more than the 12 us exchange)
         pipe = world > 1 and queries_dev[0].shape[0] >= 16
@@ -332,7 +367,7 @@ def run_ours(args):
         barrier()
         ev[0].record()
         for s in range(steps):
-            sh.search_device(queries_dev[(warm + s) % len(queries_dev)], kk, pipelined=pipe)
+            last = sh.search_device(queries_dev[(warm + s) % len(queries_dev)], kk, pipelined=pipe)
             if s == steps - 1:
                 sh.wait_results()  # the last event must cover the last batch's exchange + merge
             ev[s + 1].record()
@@ -343,7 +378,7 @@ def run_ours(args):
         prof = sh.index.profile(reset=True)
         prof["device_uncertified_all_ranks"] = allsum(prof["device_uncertified"])
         sh.index.set_profiling(False)
-        return total_ms, step_ms, prof, clocks
+        return total_ms, step_ms, prof, clocks, last
 
     def e2e_call(q, kk):
         if world == 1:
@@ -453,7 +488,6 @@ def run_ours(args):
         blk_dev = shp.search_device(d_pq, k, pipelined=world > 1)
         shp.wait_results()
         torch.cuda.synchronize()
-        from dawnsearch_b200.sharded import ResultBlock
         dl, dd, dc = ResultBlock(64, k).views(blk_dev.cpu())
         pprof = shp.index.profile()
         dev_unc = allsum(pprof["device_uncertified"])
@@ -490,7 +524,7 @@ def run_ours(args):
     if args.latency_steps > 0 and B != 1:
         q1_host = [pool_host[0][i:i + 1] for i in range(min(B, 16))]
         q1_dev = [pool_dev[0][i:i + 1] for i in range(min(B, 16))]
-        t_ms, s_ms, p1, _ = timed_device(q1_dev, k, args.latency_steps, 20)
+        t_ms, s_ms, p1, _, _ = timed_device(q1_dev, k, args.latency_steps, 20)
         e_s, l1 = timed_e2e(q1_host, k, args.latency_steps, 20)
         l1s = sorted(l1)
         batch1 = {"qps_device": args.latency_steps / (t_ms / 1e3), "qps_e2e": args.latency_steps / e_s,
@@ -499,7 +533,8 @@ def run_ours(args):
                   "roofline": roofline_of(p1, 1, peaks)}
 
     # ---- main workload -------------------------------------------------------------------
-    total_ms, step_ms, prof, clocks = timed_device(pool_dev, k, K, W, sample_clocks=True)
+    total_ms, step_ms, prof, clocks, last_block = timed_device(pool_dev, k, K, W, sample_clocks=True)
+    last_step = [a.numpy() for a in ResultBlock(B, k).views(last_block.cpu())] if args.dump_outputs and rank == 0 else None
     value = B * K / (total_ms / 1e3)
     e2e_esc[0] = 0
     e2e_s, lat = timed_e2e(pool_host, k, K, min(W, 3))
@@ -510,7 +545,7 @@ def run_ours(args):
     fp16_tiles = None
     if shadow and prof.get("shadow_batches"):
         sh.index.set_option("shadow_i8", 0)
-        t_ms, _, pf16, _ = timed_device(pool_dev, k, min(K, 5), 2)
+        t_ms, _, pf16, _, _ = timed_device(pool_dev, k, min(K, 5), 2)
         sh.index.set_option("shadow_i8", 1)
         fp16_tiles = {"value": B * min(K, 5) / (t_ms / 1e3), "unit": "queries/s", "ms_per_step": t_ms / min(K, 5), "steps": min(K, 5),
                       "note": "option shadow_i8 off: gemm_topk_kernel (tcgen05 kind::f16 tiles straight from the fp16 rows)",
@@ -529,7 +564,7 @@ def run_ours(args):
         for item in args.sweep.split(","):
             sb, sk = (int(x) for x in item.split(":")) if ":" in item else (int(item), k)
             q = [torch.from_numpy(O.make_queries(SEED, SEED + 5, sb, args.rows)).to(dev)]
-            t_ms, _, p, _ = timed_device(q, sk, 10, 3)
+            t_ms, _, p, _, _ = timed_device(q, sk, 10, 3)
             ms = t_ms / 10
             ent = {"batch": sb, "k": sk, "qps": sb / (ms / 1e3), "ms_per_step": ms,
                    "finalize_ms": p["finalize_ms"] / max(int(p["finalize_launches"]), 1)}
@@ -587,6 +622,8 @@ def run_ours(args):
         if world == 1 and not args.no_cpu_baseline:
             r = cpu_arm(args, steps=2, warmup=1, rows_total=args.rows, budget_s=20.0)
             line["cpu_baseline"] = {kk: r[kk] for kk in ("value", "unit", "cores", "kind", "sample")}
+        if last_step:
+            dump_outputs(args.dump_outputs, *last_step)
         print_json(line)
     sh.close()
     if world > 1:
@@ -648,24 +685,24 @@ def run_multi(args):
         t0 = time.perf_counter()
         for s_ in range(steps):
             t1 = time.perf_counter()
-            m.search_batch(queries[(warm + s_) % len(queries)], k)
+            last = m.search_batch(queries[(warm + s_) % len(queries)], k)
             lat.append((time.perf_counter() - t1) * 1e3)
             st = m.stats()
             dev_ms.append(st["last_search_ms"] + st["last_exchange_ms"])
             xch_ms.append(st["last_exchange_ms"])
-        return time.perf_counter() - t0, lat, dev_ms, xch_ms
+        return time.perf_counter() - t0, lat, dev_ms, xch_ms, last
 
     out_modes = {}
     for name, mode in ((("nccl", 2), ("peer", 1)) if G > 1 else (("peer", 1),)):
         m.set_option("exchange", mode)
         q1 = [pool[0][i:i + 1] for i in range(min(B, 16))]
-        w1, l1, d1, x1 = timed(q1, max(args.latency_steps, 20), 20)
+        w1, l1, d1, x1, _ = timed(q1, max(args.latency_steps, 20), 20)
         out_modes[name] = {"batch1_e2e_p50_ms": statistics.median(l1), "batch1_e2e_p99_ms": sorted(l1)[int(0.99 * len(l1))],
                            "batch1_device_p50_ms": statistics.median(d1), "batch1_exchange_merge_p50_ms": statistics.median(x1)}
     m.set_option("exchange", 0)
     sampler = ClockSampler(0)
     sampler.start()
-    wall, lat, dev_ms, xch_ms = timed(pool, K, W)
+    wall, lat, dev_ms, xch_ms, last_step = timed(pool, K, W)
     clocks = sampler.stop()
     st = m.stats()
     probe = m.search_batch(pool[0], k)
@@ -696,6 +733,8 @@ def run_multi(args):
                      "traffic": None, "corpus_stream_gbps_per_gpu": args.rows / G * row_bytes / (statistics.median(dev_ms) / 1e3) / 1e9},
         "clocks": clocks, "parity_check": parity,
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *last_step)
     print_json(line)
     m.close()
 
