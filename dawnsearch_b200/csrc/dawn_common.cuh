@@ -92,7 +92,8 @@ cudaError_t launch_gather_f32(const __half *corpus, const uint32_t *rows, size_t
                               cudaStream_t s);
 // labels[i] = first + i (synthetic corpora: label = row + 1, like SQLite rowids, search_provider.rs:275)
 cudaError_t launch_iota_labels(uint64_t *dst, uint64_t first, size_t n, cudaStream_t s);
-cudaError_t launch_shadow_quantize(const __half *corpus, uint8_t *arena, size_t first, size_t n, uint32_t *kappa_bits, cudaStream_t s);
+cudaError_t launch_shadow_quantize(const __half *corpus, uint8_t *arena, size_t first, size_t n, int group_rows,
+                                   uint32_t *kappa_bits, cudaStream_t s);
 cudaError_t launch_truncate_by_limit(const float *dist, uint32_t *counts, size_t batch, size_t k, float limit, cudaStream_t s);
 
 struct ScanLaunch {

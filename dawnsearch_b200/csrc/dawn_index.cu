@@ -186,6 +186,7 @@ struct dawn_index {
     std::atomic<int64_t> i8_tensor_min_batch{16};
     std::atomic<int64_t> i8_tensor_chunk_rows{4 << 20};
     std::atomic<int64_t> shadow_i8{0};  // 1 = keep an int8 shadow of an fp16 corpus (+388 B per row) and filter on it
+    std::atomic<int64_t> shadow_group_rows{32};  // rows sharing one scale in the shadow (1 or 32, shadow_quantize_kernel)
     std::atomic<int64_t> shadow_big_k_rows{40000000};  // compute-bound batches with k > 32 take the shadow only from this many rows on
     std::atomic<int64_t> shadow_single_rows{6000000};  // with a shadow: from this many rows on, single queries take it too
     std::atomic<int64_t> i8_native{1};  // 1 = tcgen05 kind::i8 straight from the int8 arena, 0 = dequantise to fp16 tiles
@@ -549,7 +550,8 @@ int ensure_shadow(dawn_index *idx) {
         idx->shadow_kappa = 0.f;
     }
     const size_t first = idx->shadow_rows;
-    CK(idx, launch_shadow_quantize(idx->corpus, idx->shadow, first, n - first, idx->d_shadow_kappa, idx->stream));
+    CK(idx, launch_shadow_quantize(idx->corpus, idx->shadow, first, n - first, (int)idx->shadow_group_rows, idx->d_shadow_kappa,
+                                   idx->stream));
     uint32_t bits = 0;
     CK(idx, cudaMemcpyAsync(&bits, idx->d_shadow_kappa, 4, cudaMemcpyDeviceToHost, idx->stream));
     CK(idx, cudaStreamSynchronize(idx->stream));
@@ -1931,6 +1933,16 @@ int dawn_index_set_option(dawn_index *idx, const char *key, int64_t value) {
     else if (!strcmp(key, "i8_tensor_chunk_rows")) idx->i8_tensor_chunk_rows = value < 65536 ? 65536 : value;
     else if (!strcmp(key, "i8_native")) idx->i8_native = value;
     else if (!strcmp(key, "shadow_i8")) idx->shadow_i8 = value;
+    else if (!strcmp(key, "shadow_group_rows")) {
+        if (value != 1 && value != 32) return fail(DAWN_ERR_INVALID, "shadow_group_rows must be 1 or 32, not %lld", (long long)value);
+        std::lock_guard<std::mutex> lk(idx->mu);
+        if (idx->shadow_group_rows != value) {  // the shadow is rebuilt with the new scales before the next search
+            std::unique_lock<std::shared_mutex> wr(idx->corpus_mu);
+            wait_device_searches(idx);
+            drop_shadow(idx);
+            idx->shadow_group_rows = value;
+        }
+    }
     else if (!strcmp(key, "shadow_single_rows")) idx->shadow_single_rows = value;
     else if (!strcmp(key, "shadow_big_k_rows")) idx->shadow_big_k_rows = value;
     else return fail(DAWN_ERR_INVALID, "unknown option '%s'", key);
@@ -2212,65 +2224,108 @@ cudaError_t launch_verify_rows(const void *arena, int scalar, size_t first, size
 }  // namespace
 
 namespace dawn {
-// int8 shadow of fp16 rows: per-row scale = absmax / 127, x8 = rint(x16 / scale), written in the blocked int8 layout the
-// int8 kernels read (8 rows x 384 B + 8 f32 scales per 3104-byte block).  One warp per row.  kappa_bits collects
-// max ||x16 / s - x8|| over the rows (<= sqrt(384) / 2 = 9.8 in theory, ~5.7-6.3 on real rows): the filter's rigorous
-// bound on a row's own quantisation error is ||q|| * kappa * s_row.
+// int8 shadow of fp16 rows: x8 = rint(x16 / s), written in the blocked int8 layout the int8 kernels read (8 rows x 384 B +
+// 8 f32 scales per 3104-byte block).  With group_rows = 32 every row of a group of 32 rows (aligned to the absolute row
+// index) gets the group's scale s = max absmax / 127: a group is exactly one 32-column chunk of gemm_i8_topk_kernel's
+// epilogue, whose first filter level multiplies the chunk's largest HI by its largest scale, so with one scale per chunk that
+// test is as tight as the per-element test.  Per-row scales (group_rows = 1) spread from 0.87x to 1.17x of the median and
+// make that level 12-20x looser (tools/shadow_filter_model.py).  The price is a coarser step for the rows of a group with a
+// smaller absmax: ~8-10 % more filter survivors.
+// Only rows [first, first + n) are written and only they enter their group's maximum: rows below `first` may already be read
+// by searches in flight, so a group that straddles an append keeps its old rows' scale and its new rows get their own.
+// The chunk test takes the largest scale of the chunk, so such a chunk stays rigorous, only looser.
+// Zero rows and rows with inf / NaN (which cannot be a hit of a normalised query) are stored as zeros under the group's scale
+// and are left out of its maximum; a group of nothing but such rows gets scale 1.
+// One block of 8 warps per group, 4 rows per warp.  kappa_bits collects max ||x16 / s - x8|| over the rows with the stored s
+// (<= sqrt(384) / 2 = 9.8 for any s >= absmax / 127, ~5.7-6.3 on real rows): the filter's rigorous bound on a row's own
+// quantisation error is ||q|| * kappa * s_row.
+constexpr int kShadowGroupRows = 32;
 __global__ void __launch_bounds__(256) shadow_quantize_kernel(const __half *__restrict__ corpus, uint8_t *__restrict__ arena,
-                                                              size_t first, size_t n, uint32_t *__restrict__ kappa_bits) {
-    const int lane = threadIdx.x & 31;
-    const size_t warps = (size_t)gridDim.x * (blockDim.x >> 5);
+                                                              size_t first, size_t n, int group_rows,
+                                                              uint32_t *__restrict__ kappa_bits) {
+    __shared__ float s_amax[8];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const size_t end = first + n;
+    const size_t g_end = (end + kShadowGroupRows - 1) / kShadowGroupRows;
     float kmax = 0.f;
-    for (size_t r = (size_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); r < n; r += warps) {
-        const size_t row = first + r;
-        const uint2 *src = reinterpret_cast<const uint2 *>(corpus + row * kDim) + lane * 3;  // 12 halfs per lane
-        float x[12];
-        float amax = 0.f;
+    for (size_t g = first / kShadowGroupRows + blockIdx.x; g < g_end; g += gridDim.x) {
+        float amax[4], wmax = 0.f;
 #pragma unroll
-        for (int j = 0; j < 3; j++) {
-            const uint2 u = __ldg(src + j);
-            const __half2 *h = reinterpret_cast<const __half2 *>(&u);
-            const float2 a = __half22float2(h[0]), b = __half22float2(h[1]);
-            x[4 * j] = a.x, x[4 * j + 1] = a.y, x[4 * j + 2] = b.x, x[4 * j + 3] = b.y;
-        }
+        for (int i = 0; i < 4; i++) {
+            const size_t row = g * kShadowGroupRows + warp + 8 * i;
+            float m = 0.f;
+            if (row >= first && row < end) {
+                const uint2 *src = reinterpret_cast<const uint2 *>(corpus + row * kDim) + lane * 3;  // 12 halfs per lane
 #pragma unroll
-        for (int j = 0; j < 12; j++) amax = fmaxf(amax, fabsf(x[j]));
-#pragma unroll
-        for (int off = 16; off > 0; off >>= 1) amax = fmaxf(amax, __shfl_xor_sync(0xffffffffu, amax, off));
-        if (!(amax < INFINITY)) amax = 0.f;  // a row with inf / NaN cannot be a hit of a normalised query: stored as zeros
-        const float sc = amax > 0.f ? __fdiv_rn(amax, 127.0f) : 1.0f;
-        uint32_t packed[3];
-        float err2 = 0.f;
-#pragma unroll
-        for (int j = 0; j < 3; j++) {
-            uint32_t w = 0;
-#pragma unroll
-            for (int e = 0; e < 4; e++) {
-                const float v = amax > 0.f ? x[4 * j + e] : 0.f;
-                const float t = __fdiv_rn(v, sc);
-                const int qv = max(-127, min(127, (int)rintf(t)));
-                const float d = t - (float)qv;
-                err2 = fmaf(d, d, err2);
-                w |= ((uint32_t)(qv & 0xff)) << (8 * e);
+                for (int j = 0; j < 3; j++) {
+                    const uint2 u = __ldg(src + j);
+                    const float2 a = __half22float2(*reinterpret_cast<const __half2 *>(&u.x));
+                    const float2 b = __half22float2(*reinterpret_cast<const __half2 *>(&u.y));
+                    m = fmaxf(fmaxf(m, fmaxf(fabsf(a.x), fabsf(a.y))), fmaxf(fabsf(b.x), fabsf(b.y)));
+                }
             }
-            packed[j] = w;
-        }
 #pragma unroll
-        for (int off = 16; off > 0; off >>= 1) err2 += __shfl_xor_sync(0xffffffffu, err2, off);
-        uint32_t *dst = reinterpret_cast<uint32_t *>(arena + i8_row_offset((uint32_t)row)) + lane * 3;
-        dst[0] = packed[0], dst[1] = packed[1], dst[2] = packed[2];
-        if (lane == 0) *reinterpret_cast<float *>(arena + i8_scale_offset((uint32_t)row)) = sc;
-        kmax = fmaxf(kmax, sqrtf(err2) * 1.00001f);
+            for (int off = 16; off > 0; off >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, off));
+            if (!(m < INFINITY)) m = 0.f;
+            amax[i] = m;
+            wmax = fmaxf(wmax, m);
+        }
+        if (group_rows > 1) {
+            if (lane == 0) s_amax[warp] = wmax;
+            __syncthreads();
+            wmax = s_amax[0];
+#pragma unroll
+            for (int w = 1; w < 8; w++) wmax = fmaxf(wmax, s_amax[w]);
+            __syncthreads();  // s_amax is rewritten for the next group
+        }
+        // second pass over the same rows (L1 / L2 hits): keeping all four in registers through the divisions spills
+#pragma unroll 1
+        for (int i = 0; i < 4; i++) {
+            const size_t row = g * kShadowGroupRows + warp + 8 * i;
+            if (row < first || row >= end) continue;
+            const float ra = i == 0 ? amax[0] : i == 1 ? amax[1] : i == 2 ? amax[2] : amax[3];
+            const float m = group_rows > 1 ? wmax : ra;
+            const float sc = m > 0.f ? __fdiv_rn(m, 127.0f) : 1.0f;
+            const uint2 *src = reinterpret_cast<const uint2 *>(corpus + row * kDim) + lane * 3;
+            uint32_t packed[3];
+            float err2 = 0.f;
+#pragma unroll
+            for (int j = 0; j < 3; j++) {
+                const uint2 u = __ldg(src + j);
+                const float2 a = __half22float2(*reinterpret_cast<const __half2 *>(&u.x));
+                const float2 b = __half22float2(*reinterpret_cast<const __half2 *>(&u.y));
+                const float xs[4] = {a.x, a.y, b.x, b.y};
+                uint32_t w = 0;
+#pragma unroll
+                for (int e = 0; e < 4; e++) {
+                    const float v = ra > 0.f ? xs[e] : 0.f;
+                    const float t = __fdiv_rn(v, sc);
+                    const int qv = max(-127, min(127, (int)rintf(t)));
+                    const float d = t - (float)qv;
+                    err2 = fmaf(d, d, err2);
+                    w |= ((uint32_t)(qv & 0xff)) << (8 * e);
+                }
+                packed[j] = w;
+            }
+#pragma unroll
+            for (int off = 16; off > 0; off >>= 1) err2 += __shfl_xor_sync(0xffffffffu, err2, off);
+            uint32_t *dst = reinterpret_cast<uint32_t *>(arena + i8_row_offset((uint32_t)row)) + lane * 3;
+            dst[0] = packed[0], dst[1] = packed[1], dst[2] = packed[2];
+            if (lane == 0) *reinterpret_cast<float *>(arena + i8_scale_offset((uint32_t)row)) = sc;
+            kmax = fmaxf(kmax, sqrtf(err2) * 1.00001f);
+        }
     }
     if (lane == 0 && kmax > 0.f) atomicMax(kappa_bits, __float_as_uint(kmax));
 }
 
-cudaError_t launch_shadow_quantize(const __half *corpus, uint8_t *arena, size_t first, size_t n, uint32_t *kappa_bits,
-                                   cudaStream_t s) {
+cudaError_t launch_shadow_quantize(const __half *corpus, uint8_t *arena, size_t first, size_t n, int group_rows,
+                                   uint32_t *kappa_bits, cudaStream_t s) {
     if (n == 0) return cudaSuccess;
-    size_t blocks = (n + 7) / 8;
-    if (blocks > 148 * 32) blocks = 148 * 32;
-    shadow_quantize_kernel<<<(unsigned)blocks, 256, 0, s>>>(corpus, arena, first, n, kappa_bits);
+    if (group_rows != 1 && group_rows != kShadowGroupRows) return cudaErrorInvalidValue;
+    const size_t groups = (first + n + kShadowGroupRows - 1) / kShadowGroupRows - first / kShadowGroupRows;
+    size_t blocks = groups;
+    if (blocks > 148 * 8) blocks = 148 * 8;
+    shadow_quantize_kernel<<<(unsigned)blocks, 256, 0, s>>>(corpus, arena, first, n, group_rows, kappa_bits);
     return cudaGetLastError();
 }
 

@@ -86,6 +86,27 @@ struct I8Smem {  // offsets from the 1024-aligned base
     // barriers (8 B each): full[6], empty[6], tmem_full[2], tmem_empty[2], a_full, a_free, scale_full[8]; then tmem ptr
 };
 
+#ifdef DAWN_COUNT_SLOW_PATH
+// Measurement build only (make EXTRA=-DDAWN_COUNT_SLOW_PATH; tools/slow_path_count.py reads it): per launch of
+// gemm_i8_topk_kernel, the epilogue's warp-chunks (32 queries x 32 columns) that went on to levels 2 and 3 (examine())
+// and all warp-chunks processed.  slow_path_log_kernel, enqueued after each launch, moves the sums into a log.
+__device__ unsigned long long g_slow_acc[2];
+constexpr int kSlowLogCap = 4096;
+__device__ unsigned long long g_slow_log[kSlowLogCap][4];  // {slow warp-chunks, warp-chunks, tiles of the launch, queries}
+__device__ unsigned int g_slow_log_n;
+__global__ void slow_path_log_kernel(uint32_t tiles, int n_queries) {
+    const unsigned int i = g_slow_log_n;
+    if (i < (unsigned int)kSlowLogCap) {
+        g_slow_log[i][0] = g_slow_acc[0];
+        g_slow_log[i][1] = g_slow_acc[1];
+        g_slow_log[i][2] = tiles;
+        g_slow_log[i][3] = (unsigned long long)n_queries;
+        g_slow_log_n = i + 1;
+    }
+    g_slow_acc[0] = g_slow_acc[1] = 0ull;
+}
+#endif
+
 __device__ __noinline__ void flush_staged_i8(uint32_t stage_smem, int col, uint32_t n, uint2 *__restrict__ log_q,
                                              uint32_t *__restrict__ cnt_q, uint32_t *__restrict__ overflow_q, int cap) {
     uint32_t slot = atomicAdd(cnt_q, n);
@@ -287,6 +308,9 @@ gemm_i8_topk_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_con
         const uint32_t gmax_smem = base + I8Smem::groupmax_off + (uint32_t)(warp - 4) * 128u;
         uint32_t n_st = 0;
         uint32_t tile_ctr = 0;
+#ifdef DAWN_COUNT_SLOW_PATH
+        uint32_t n_slow = 0, n_wchunks = 0;
+#endif
         const uint32_t tempty_lead0 = CG == 2 ? mapa_rank(tempty_bar(0), 0) : 0u;
         const uint32_t tempty_lead1 = CG == 2 ? mapa_rank(tempty_bar(1), 0) : 0u;
         for (uint32_t u = unit_first; u < n_units; u += unit_stride) {
@@ -369,6 +393,10 @@ gemm_i8_topk_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_con
                     const int mm = max(max(max(m[0], m[1]), max(m[2], m[3])), max(max(m[4], m[5]), max(m[6], m[7])));
                     const float sm_c = __shfl_sync(0xffffffffu, smax, 8 * c);
                     const bool hit = q_valid && (!thr_pos || (__int2float_rn(mm) + cq) * sm_c >= thr);
+#ifdef DAWN_COUNT_SLOW_PATH
+                    n_slow += __any_sync(0xffffffffu, hit) ? 1u : 0u;
+                    n_wchunks++;
+#endif
                     if (hit) examine(v, m, c);
                     __syncwarp();
                 };
@@ -401,6 +429,12 @@ gemm_i8_topk_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_con
             }
             __syncwarp();
         }
+#ifdef DAWN_COUNT_SLOW_PATH
+        if (lane == 0) {
+            atomicAdd(&g_slow_acc[0], (unsigned long long)n_slow);
+            atomicAdd(&g_slow_acc[1], (unsigned long long)n_wchunks);
+        }
+#endif
     }
 
     tc_fence_before();
@@ -864,6 +898,9 @@ cudaError_t launch_gemm_search_i8(const GemmSearchI8 &p, cudaStream_t s) {
             e = launch_round<1>(p.grid, s, tq, tx, ts, (uint32_t)begin, (uint32_t)end, (uint32_t)p.n_rows, (uint32_t)total_tiles,
                                 (uint32_t)mult, n_qtiles, p.n_queries, (int)chunk, thr, cnt, log, overflow, arrive, cq);
         if (e != cudaSuccess) return e;
+#ifdef DAWN_COUNT_SLOW_PATH
+        slow_path_log_kernel<<<1, 1, 0, s>>>((uint32_t)(end - begin), p.n_queries);
+#endif
         const bool last = end >= total_tiles;
         select_i8_kernel<<<qp, kSelThreads, 0, s>>>(log, cnt, kept, thr, overflow, kSelCap, p.kprime, p.arena, p.queries,
                                                     p.n_queries, s1, e1, p.limit_score, p.eps_scale, p.labels,
@@ -879,3 +916,19 @@ cudaError_t launch_gemm_search_i8(const GemmSearchI8 &p, cudaStream_t s) {
 }
 
 }  // namespace dawn
+
+#ifdef DAWN_COUNT_SLOW_PATH
+// The measurement build's log on the current device: copies up to `cap` entries of 4 u64 into out, returns the number logged
+// (-1 on a CUDA error); reset != 0 then empties it.
+extern "C" int dawn_debug_slow_path_log(unsigned long long *out, int cap, int reset) {
+    unsigned int n = 0;
+    if (cudaDeviceSynchronize() != cudaSuccess || cudaMemcpyFromSymbol(&n, dawn::g_slow_log_n, sizeof n) != cudaSuccess) return -1;
+    const int m = (int)n < cap ? (int)n : cap;
+    if (m > 0 && cudaMemcpyFromSymbol(out, dawn::g_slow_log, (size_t)m * 4 * sizeof(unsigned long long)) != cudaSuccess) return -1;
+    if (reset) {
+        const unsigned int zero = 0;
+        if (cudaMemcpyToSymbol(dawn::g_slow_log_n, &zero, sizeof zero) != cudaSuccess) return -1;
+    }
+    return (int)n;
+}
+#endif

@@ -285,6 +285,9 @@ int dawn_index_set_profiling(dawn_index *idx, int enable);
  * "shadow_i8" (0): 1 = an fp16 corpus also keeps an int8 copy of itself (+388 B per row, built lazily before a search) and
  * batches that would take the fp16 tensor-core path are FILTERED on the copy by the int8 tensor cores instead -- half the
  * HBM bytes, twice the MMA rate -- while every candidate is re-scored on the fp16 rows: results stay bit-identical.
+ * "shadow_group_rows" (32; 1 or 32): rows of the copy that share one scale, in groups aligned to the row index.  32 makes the
+ * filter's first level as tight as its per-element test; 1 = a scale per row.  A change drops the copy (it waits for searches
+ * in flight) and the next search rebuilds it.  Results are the same either way.
  * "shadow_single_rows" (6M): with a shadow, from this many rows on even a single query takes that path (388 B per row
  * instead of the scan's 768 B).  "shadow_big_k_rows" (40M): batches of >= 128 queries with k > 32 take it only from this many
  * rows on (below, the exact re-scores of k + 4 candidates per round cost more than the int8 tiles save).
