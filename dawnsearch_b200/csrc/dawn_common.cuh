@@ -254,4 +254,25 @@ struct GemmSearchI8 {
 cudaError_t launch_gemm_search_i8(const GemmSearchI8 &p, cudaStream_t s);
 size_t gemm_i8_workspace_bytes(int n_queries);
 
+// dawn_index_remove_batch (remove.cu).  mark: hash the m requested labels (d_req, device) and flag every row of
+// labels[0, n) whose label is among them; meta_out (host) receives {r = rows flagged, h = flagged rows below n - r}.
+// pair: holes[i] = i-th flagged row below n - r, donors[i] = i-th unflagged row in [n - r, n), i < h.  Both read the
+// scratch of remove_scratch_bytes(m, n) that mark filled.
+size_t remove_scratch_bytes(size_t m, size_t n);
+cudaError_t launch_remove_mark(const uint64_t *d_req, size_t m, const uint64_t *labels, size_t n, void *scratch, uint32_t *meta_out,
+                               cudaStream_t s);
+cudaError_t launch_remove_pair(const void *scratch, size_t m, size_t n, uint32_t r, uint32_t h, uint32_t *holes, uint32_t *donors,
+                               cudaStream_t s);
+struct RemoveMove {
+    const uint32_t *holes, *donors;
+    size_t n_pairs;
+    uint8_t *arena;     // fp16 rows, or the blocked int8 arena when i8
+    int i8;
+    float *corpus32;    // DAWN_SCALAR_F32 only, else null
+    uint8_t *shadow;    // the int8 shadow of an fp16 corpus, or null
+    uint64_t *labels;
+};
+// move: copy every row, scale and label of donors[i] into holes[i].
+cudaError_t launch_remove_move(const RemoveMove &p, cudaStream_t s);
+
 }  // namespace dawn

@@ -1323,6 +1323,88 @@ int bulk_add(dawn_index *idx, const uint64_t *labels, const float *vectors, size
     return DAWN_OK;
 }
 
+// ---- remove: compaction (remove.cu) ----------------------------------------------------------------
+// idx->mu held.  Staged adds are flushed and every row is norm-checked and, when a shadow exists, quantised BEFORE the rows
+// are paired: a donor moves below the new size, and a row that had not passed the gate scan or the quantiser by then would
+// sit below both watermarks forever.  Mark and pair only read the label table, which nothing else writes while mu is held,
+// so they run while searches go on; the moves and the new size are published under the exclusive corpus lock after every
+// search in flight has finished, like a reallocation (grow_physical).
+// A moved shadow row keeps its own scale: the kappa bound is per row, and the filter's chunk test takes the largest scale of
+// the chunk's columns, so a 32-row group that receives a donor stays rigorous, only possibly looser -- like a group split by
+// an append.  At most one group per removed row becomes mixed.  The norm statistics are left as they are: they bound a
+// superset of the stored rows, so the certificate stays sound; dawn_index_verify rescans from zero and tightens them.
+int remove_rows(dawn_index *idx, const uint64_t *req, size_t m, size_t *removed) {
+    *removed = 0;
+    int rc;
+    if ((rc = flush_staged(idx)) || (rc = ensure_norms_checked(idx)) || (rc = ensure_shadow(idx))) return rc;
+    const size_t n = idx->size;
+    if (n == 0) return DAWN_OK;
+    cudaStream_t s = idx->stream;
+    const size_t req_bytes = (m * sizeof(uint64_t) + 255) / 256 * 256;
+    uint8_t *scratch = nullptr;
+    uint32_t *pairs = nullptr;
+    const size_t scratch_bytes = req_bytes + remove_scratch_bytes(m, n);
+    if (cudaMallocAsync(reinterpret_cast<void **>(&scratch), scratch_bytes, s) != cudaSuccess) {
+        cudaGetLastError();
+        return fail(DAWN_ERR_CAPACITY, "cannot allocate %zu bytes of HBM to remove %zu labels", scratch_bytes, m);
+    }
+    auto release = [&] {
+        cudaFreeAsync(scratch, s);
+        if (pairs) cudaFreeAsync(pairs, s);
+    };
+    uint32_t meta[2] = {0, 0};
+    cudaError_t e = cudaMemcpyAsync(scratch, req, m * sizeof(uint64_t), cudaMemcpyHostToDevice, s);
+    if (e == cudaSuccess) e = launch_remove_mark(reinterpret_cast<const uint64_t *>(scratch), m, idx->labels, n, scratch + req_bytes, meta, s);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+    const uint32_t r = meta[0], h = meta[1];
+    if (e == cudaSuccess && h > 0) {
+        if (cudaMallocAsync(reinterpret_cast<void **>(&pairs), 2 * (size_t)h * sizeof(uint32_t), s) != cudaSuccess) {
+            cudaGetLastError();
+            pairs = nullptr;
+            release();
+            return fail(DAWN_ERR_CAPACITY, "cannot allocate the %u row pairs of a remove", h);
+        }
+        e = launch_remove_pair(scratch + req_bytes, m, n, r, h, pairs, pairs + h, s);
+    }
+    if (e != cudaSuccess || r == 0) {
+        release();
+        CK(idx, e);
+        return DAWN_OK;
+    }
+    {
+        std::unique_lock<std::shared_mutex> wr(idx->corpus_mu);
+        wait_device_searches(idx);
+        // A shadow that lags the corpus (it is only extended from 65536 rows on, and not while the option is off) would hand
+        // unquantised donor rows to holes below its watermark: drop it instead, the next search that wants it rebuilds it.
+        if (idx->shadow.load() && idx->shadow_rows < n) drop_shadow(idx);
+        RemoveMove mv;
+        mv.holes = pairs;
+        mv.donors = pairs ? pairs + h : nullptr;
+        mv.n_pairs = h;
+        mv.arena = reinterpret_cast<uint8_t *>(idx->corpus);
+        mv.i8 = idx->scalar == DAWN_SCALAR_I8;
+        mv.corpus32 = idx->corpus32;
+        mv.shadow = idx->shadow.load();
+        mv.labels = idx->labels;
+        e = launch_remove_move(mv, s);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+        if (e == cudaSuccess) {
+            const size_t left = n - r;
+            idx->size = left;
+            if (idx->shadow_rows > left) idx->shadow_rows = left;
+            if (idx->norm_checked > left) idx->norm_checked = left;
+        }
+    }
+    release();
+    CK(idx, e);
+    {
+        std::lock_guard<std::mutex> lk(idx->prof_mu);
+        idx->prof.kernel_launches += h > 0 ? 5 : 3;
+    }
+    *removed = r;
+    return DAWN_OK;
+}
+
 }  // namespace
 
 // ------------------------------------------------------------------------------ C ABI
@@ -1502,6 +1584,26 @@ int dawn_index_add_synthetic(dawn_index *idx, uint64_t seed, uint64_t first_row,
         idx->prof.kernel_launches += 2;
     }
     return DAWN_OK;
+}
+
+// The rows of every listed label are compacted out of the device corpus (remove_rows); capacity is kept.
+int dawn_index_remove_batch(dawn_index *idx, const uint64_t *labels, size_t n, size_t *removed_out) {
+    if (removed_out) *removed_out = 0;
+    if (!idx) return fail(DAWN_ERR_INVALID, "null index handle");
+    if (n > 0 && !labels) return fail(DAWN_ERR_INVALID, "labels is null");
+    int rc = check_alive(idx);
+    if (rc) return rc;
+    if (n == 0) return DAWN_OK;
+    std::lock_guard<std::mutex> lk(idx->mu);
+    size_t removed = 0;
+    rc = remove_rows(idx, labels, n, &removed);
+    if (rc) return rc;
+    if (removed_out) *removed_out = removed;
+    return DAWN_OK;
+}
+
+int dawn_index_remove(dawn_index *idx, uint64_t label, size_t *removed_out) {
+    return dawn_index_remove_batch(idx, &label, 1, removed_out);
 }
 
 int dawn_index_search_batch(dawn_index *idx, const float *queries, size_t batch, size_t k,

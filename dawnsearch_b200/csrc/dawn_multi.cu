@@ -380,6 +380,28 @@ int dawn_multi_add_synthetic(dawn_multi *m, uint64_t seed, uint64_t first_row, s
     });
 }
 
+// Adds place labels on any shard, so every shard runs the remove (concurrently); the counts are summed.
+int dawn_multi_remove_batch(dawn_multi *m, const uint64_t *labels, size_t n, size_t *removed_out) {
+    if (removed_out) *removed_out = 0;
+    if (!m || (n && !labels)) {
+        g_multi_err = !m ? "null multi handle" : "labels is null";
+        return DAWN_ERR_INVALID;
+    }
+    if (n == 0) return DAWN_OK;
+    std::lock_guard<std::mutex> lk(m->mu);
+    std::vector<size_t> removed(m->shards.size(), 0);
+    size_t *counts = removed.data();
+    int rc = run_all(m, [=](Shard *s, size_t g) -> int { return dawn_index_remove_batch(s->idx, labels, n, counts + g); });
+    // a shard that failed reports 0; the others have removed their rows, and the count says so even when rc != 0
+    if (removed_out)
+        for (size_t r : removed) *removed_out += r;
+    return rc;
+}
+
+int dawn_multi_remove(dawn_multi *m, uint64_t label, size_t *removed_out) {
+    return dawn_multi_remove_batch(m, &label, 1, removed_out);
+}
+
 // distance_limit (NaN = none): every shard pushes the limit down into its kernels and cuts its counts on the device, so
 // only hits with distance < limit are exchanged and merged (UdpPacket::Search.distance_limit, src/net/udp_packets.rs:29-39;
 // filter src/net/udp_service.rs:196-199).

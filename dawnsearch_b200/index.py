@@ -162,6 +162,8 @@ def load_library() -> C.CDLL:
     L.dawn_index_reserve.argtypes = [_vp, C.c_size_t]
     L.dawn_index_add.argtypes = [_vp, C.c_uint64, _vp]
     L.dawn_index_add_batch.argtypes = [_vp, _vp, _vp, C.c_size_t]
+    L.dawn_index_remove.argtypes = [_vp, C.c_uint64, _vp]
+    L.dawn_index_remove_batch.argtypes = [_vp, _vp, C.c_size_t, _vp]
     L.dawn_index_search.argtypes = [_vp, _vp, C.c_size_t, _vp, _vp, _vp]
     L.dawn_index_search_batch.argtypes = [_vp, _vp, C.c_size_t, C.c_size_t, _vp, _vp, _vp]
     L.dawn_index_search_device.argtypes = [_vp, _vp, C.c_size_t, C.c_size_t, _vp, _vp, _vp, _vp, _vp]
@@ -207,6 +209,8 @@ def load_library() -> C.CDLL:
     L.dawn_multi_add.argtypes = [_vp, C.c_uint64, _vp]
     L.dawn_multi_add_batch.argtypes = [_vp, _vp, _vp, C.c_size_t]
     L.dawn_multi_add_synthetic.argtypes = [_vp, C.c_uint64, C.c_uint64, C.c_size_t]
+    L.dawn_multi_remove.argtypes = [_vp, C.c_uint64, _vp]
+    L.dawn_multi_remove_batch.argtypes = [_vp, _vp, C.c_size_t, _vp]
     L.dawn_multi_search.argtypes = [_vp, _vp, C.c_size_t, _vp, _vp, _vp]
     L.dawn_multi_search_batch.argtypes = [_vp, _vp, C.c_size_t, C.c_size_t, _vp, _vp, _vp]
     L.dawn_multi_search_batch_limit.argtypes = [_vp, _vp, C.c_size_t, C.c_size_t, C.c_float, _vp, _vp, _vp]
@@ -279,6 +283,20 @@ class Index:
         if lab.shape[0] != v.shape[0]:
             raise DawnError(-1, "labels and vectors differ in length")
         _check(self._L.dawn_index_add_batch(self._h, _ptr(lab), _ptr(v), v.shape[0]))
+
+    def remove(self, label: int) -> int:
+        """Remove every stored vector with this label; returns how many were removed (0 if none)."""
+        n = C.c_size_t(0)
+        _check(self._L.dawn_index_remove(self._h, int(label), C.byref(n)))
+        return int(n.value)
+
+    def remove_batch(self, labels) -> int:
+        """Remove every stored vector whose label is listed (repeats and absent labels are fine); returns the rows removed.
+        An update is remove(label) followed by add(label, vector)."""
+        lab = np.ascontiguousarray(labels, dtype=np.uint64).reshape(-1)
+        n = C.c_size_t(0)
+        _check(self._L.dawn_index_remove_batch(self._h, _ptr(lab), lab.shape[0], C.byref(n)))
+        return int(n.value)
 
     def search(self, query, count: int) -> Matches:  # search_provider.rs:214
         q = np.ascontiguousarray(query, dtype=np.float32)
@@ -534,6 +552,18 @@ class MultiIndex:
 
     def add_synthetic(self, seed: int, first_row: int, n: int) -> None:
         self._check(self._L.dawn_multi_add_synthetic(self._h, seed, first_row, n))
+
+    def remove(self, label: int) -> int:
+        """Remove the label's vectors from every shard; returns the rows removed."""
+        n = C.c_size_t(0)
+        self._check(self._L.dawn_multi_remove(self._h, int(label), C.byref(n)))
+        return int(n.value)
+
+    def remove_batch(self, labels) -> int:
+        lab = np.ascontiguousarray(labels, dtype=np.uint64).reshape(-1)
+        n = C.c_size_t(0)
+        self._check(self._L.dawn_multi_remove_batch(self._h, _ptr(lab), lab.shape[0], C.byref(n)))
+        return int(n.value)
 
     def search(self, query, count: int) -> Matches:
         q = np.ascontiguousarray(query, dtype=np.float32)

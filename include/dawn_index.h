@@ -34,8 +34,8 @@
  * Threading: the reference drives its index from a single thread
  * (src/bin/dawnsearch.rs:76-78); that model works unchanged.  Beyond it, search* / get are re-entrant:
  * every host search leases its own stream + workspace (up to 8 in flight per handle), so several threads
- * may search one handle concurrently.  add* / reserve / save / load are serialised among themselves; an
- * add never waits for running searches (it appends beyond what they see), only a reallocation does.
+ * may search one handle concurrently.  add* / remove* / reserve / save / load are serialised among themselves; an
+ * add never waits for running searches (it appends beyond what they see), only a reallocation or a remove does.
  * A handle may be used from any thread; different handles are independent.
  */
 #ifndef DAWN_INDEX_H
@@ -98,6 +98,14 @@ int dawn_index_reserve(dawn_index *idx, size_t n);
  * reserve(size+1024) itself, search_provider.rs:280-283). */
 int dawn_index_add(dawn_index *idx, uint64_t label, const float *vector384);
 int dawn_index_add_batch(dawn_index *idx, const uint64_t *labels, const float *vectors, size_t n);
+/* Remove every stored row whose label is in labels[0..n) (duplicates in the list and absent labels are fine).
+ * *removed_out (may be NULL) = rows removed.  Staged adds made before the call are covered.  size() drops by the
+ * count; capacity is unchanged.  Like a reallocation, it waits for searches in flight; searches that start later
+ * see the new corpus.  Serialised with add* / reserve / save / load.  The last rows of the corpus move into the
+ * freed places (exact search does not depend on row order).  An update is a remove followed by an add.
+ * n > 0 with labels == NULL, or a NULL handle: DAWN_ERR_INVALID. */
+int dawn_index_remove_batch(dawn_index *idx, const uint64_t *labels, size_t n, size_t *removed_out);
+int dawn_index_remove(dawn_index *idx, uint64_t label, size_t *removed_out);
 
 /* Exact top-k for one / `batch` f32 queries in host memory.  Output buffers are caller
  * allocated: labels[batch*k], distances[batch*k], counts[batch]; row b's results occupy
@@ -225,6 +233,10 @@ int dawn_multi_reserve(dawn_multi *m, size_t n_total);
 int dawn_multi_add(dawn_multi *m, uint64_t label, const float *vector384);
 int dawn_multi_add_batch(dawn_multi *m, const uint64_t *labels, const float *vectors, size_t n);
 int dawn_multi_add_synthetic(dawn_multi *m, uint64_t seed, uint64_t first_row, size_t n);
+/* dawn_index_remove_batch on every shard (a label may be stored on any of them); *removed_out = the shards' counts summed.
+ * If a shard fails, the error is returned and *removed_out still counts the rows the other shards removed. */
+int dawn_multi_remove_batch(dawn_multi *m, const uint64_t *labels, size_t n, size_t *removed_out);
+int dawn_multi_remove(dawn_multi *m, uint64_t label, size_t *removed_out);
 int dawn_multi_search(dawn_multi *m, const float *query384, size_t k, uint64_t *labels_out, float *distances_out,
                       size_t *count_out);
 int dawn_multi_search_batch(dawn_multi *m, const float *queries, size_t batch, size_t k, uint64_t *labels_out,

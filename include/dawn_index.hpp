@@ -177,6 +177,17 @@ public:
         if (vectors.size() != labels.size() * EM_LEN) throw Error(DAWN_ERR_INVALID, "vectors must be labels x 384");
         check(dawn_index_add_batch(h_, labels.data(), vectors.data(), labels.size()));
     }
+    // Drop every stored vector with this label / these labels; returns the vectors removed.  Update = remove + add.
+    std::size_t remove(std::uint64_t label) const {
+        std::size_t n = 0;
+        check(dawn_index_remove(h_, label, &n));
+        return n;
+    }
+    std::size_t remove_batch(const std::vector<std::uint64_t> &labels) const {
+        std::size_t n = 0;
+        check(dawn_index_remove_batch(h_, labels.data(), labels.size(), &n));
+        return n;
+    }
     Matches search(const std::vector<float> &query, std::size_t count) const {                    // :214
         if (query.size() != EM_LEN) throw Error(DAWN_ERR_INVALID, "query must have 384 dimensions");
         Matches m;

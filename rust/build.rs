@@ -11,7 +11,7 @@ use std::{env, path::PathBuf, process::Command};
 // keep in sync with SRCS in dawnsearch_b200/csrc/Makefile (enforced by tests/test_rust_shim.py)
 const SRCS: &[&str] = &[
     "dawn_index.cu", "scan_topk.cu", "finalize.cu", "ingest.cu", "gemm_topk.cu", "gemm_i8.cu", "i8_tensor.cu",
-    "dawn_front.cu", "dawn_multi.cu",
+    "dawn_front.cu", "dawn_multi.cu", "remove.cu",
 ];
 // keep in sync with NVCCFLAGS in dawnsearch_b200/csrc/Makefile.  -ffp-contract=off matters: the host mirrors
 // of src/search/vector.rs:181-197 (dawn_front.cu) must not fuse a*b+c, Rust never does.

@@ -18,6 +18,8 @@ extern "C" {
     fn dawn_index_reserve(idx: *mut c_void, n: usize) -> c_int;
     fn dawn_index_add(idx: *mut c_void, label: u64, v: *const f32) -> c_int;
     fn dawn_index_add_batch(idx: *mut c_void, labels: *const u64, v: *const f32, n: usize) -> c_int;
+    fn dawn_index_remove(idx: *mut c_void, label: u64, removed: *mut usize) -> c_int;
+    fn dawn_index_remove_batch(idx: *mut c_void, labels: *const u64, n: usize, removed: *mut usize) -> c_int;
     fn dawn_index_search(idx: *mut c_void, q: *const f32, k: usize, labels: *mut u64, dist: *mut f32, count: *mut usize) -> c_int;
     fn dawn_index_search_batch(idx: *mut c_void, q: *const f32, batch: usize, k: usize, labels: *mut u64, dist: *mut f32, counts: *mut usize) -> c_int;
     fn dawn_index_size(idx: *const c_void) -> usize;
@@ -43,6 +45,8 @@ extern "C" {
     fn dawn_multi_reserve(m: *mut c_void, n_total: usize) -> c_int;
     fn dawn_multi_add(m: *mut c_void, label: u64, v: *const f32) -> c_int;
     fn dawn_multi_add_batch(m: *mut c_void, labels: *const u64, v: *const f32, n: usize) -> c_int;
+    fn dawn_multi_remove(m: *mut c_void, label: u64, removed: *mut usize) -> c_int;
+    fn dawn_multi_remove_batch(m: *mut c_void, labels: *const u64, n: usize, removed: *mut usize) -> c_int;
     fn dawn_multi_search(m: *mut c_void, q: *const f32, k: usize, labels: *mut u64, dist: *mut f32, count: *mut usize) -> c_int;
     fn dawn_multi_search_batch(m: *mut c_void, q: *const f32, batch: usize, k: usize, labels: *mut u64, dist: *mut f32, counts: *mut usize) -> c_int;
     fn dawn_multi_search_limit(m: *mut c_void, q: *const f32, k: usize, limit: f32, labels: *mut u64, dist: *mut f32, count: *mut usize) -> c_int;
@@ -96,6 +100,18 @@ impl Index {
     pub fn add_batch(&self, labels: &[u64], vectors: &[f32]) -> anyhow::Result<()> {      // bulk rebuild (fill_index_from_db, :127-153)
         anyhow::ensure!(vectors.len() == labels.len() * 384, "vectors must be labels.len() x 384");
         ck(unsafe { dawn_index_add_batch(self.h, labels.as_ptr(), vectors.as_ptr(), labels.len()) })
+    }
+    /// Drops every stored vector with `label` (a page that was deleted); returns how many were removed.  A re-crawled or
+    /// re-embedded page is `remove(id)` then `add(id, &v)`.
+    pub fn remove(&self, label: u64) -> anyhow::Result<usize> {
+        let mut n = 0usize;
+        ck(unsafe { dawn_index_remove(self.h, label, &mut n) })?;
+        Ok(n)
+    }
+    pub fn remove_batch(&self, labels: &[u64]) -> anyhow::Result<usize> {
+        let mut n = 0usize;
+        ck(unsafe { dawn_index_remove_batch(self.h, labels.as_ptr(), labels.len(), &mut n) })?;
+        Ok(n)
     }
     pub fn search(&self, query: &[f32], count: usize) -> anyhow::Result<Matches> {                                            // :214
         anyhow::ensure!(query.len() == 384, "query must have 384 dimensions");
@@ -193,6 +209,17 @@ impl MultiIndex {
     pub fn add_batch(&self, labels: &[u64], vectors: &[f32]) -> anyhow::Result<()> {
         anyhow::ensure!(vectors.len() == labels.len() * 384, "vectors must be labels.len() x 384");
         mck(unsafe { dawn_multi_add_batch(self.m, labels.as_ptr(), vectors.as_ptr(), labels.len()) })
+    }
+    /// Drops the label's vectors on every shard; returns how many were removed in all.
+    pub fn remove(&self, label: u64) -> anyhow::Result<usize> {
+        let mut n = 0usize;
+        mck(unsafe { dawn_multi_remove(self.m, label, &mut n) })?;
+        Ok(n)
+    }
+    pub fn remove_batch(&self, labels: &[u64]) -> anyhow::Result<usize> {
+        let mut n = 0usize;
+        mck(unsafe { dawn_multi_remove_batch(self.m, labels.as_ptr(), labels.len(), &mut n) })?;
+        Ok(n)
     }
     pub fn search(&self, query: &[f32], count: usize) -> anyhow::Result<Matches> {
         anyhow::ensure!(query.len() == 384, "query must have 384 dimensions");
