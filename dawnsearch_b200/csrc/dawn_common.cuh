@@ -80,7 +80,8 @@ __host__ __device__ inline int32_t synth_raw(uint64_t seed, uint64_t row, uint32
 
 // K1: f32 page vectors -> stored fp16 rows (round to nearest even), appended at dst.
 // Replaces the per-vector work of usearch Index::add (src/search/search_provider.rs:149,284).
-cudaError_t launch_ingest_f16(const float *src_f32, __half *dst, size_t n_rows, cudaStream_t s);
+// saturate: clamp to +-65504 instead of rounding to inf (the selection copy of DAWN_SCALAR_F32 rows)
+cudaError_t launch_ingest_f16(const float *src_f32, __half *dst, size_t n_rows, cudaStream_t s, bool saturate = false);
 // Synthetic rows [first_row, first_row+n) written straight into the corpus arena.
 cudaError_t launch_synth_f16(__half *dst, uint64_t seed, uint64_t first_row, size_t n_rows,
                              cudaStream_t s);

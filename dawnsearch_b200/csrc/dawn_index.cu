@@ -80,6 +80,7 @@ struct SearchWs {
     cudaStream_t stream = nullptr;  // owned
     size_t n_rows = 0;              // snapshot of the index size this search sees
     float eps_scale = 1.0f;         // > 1 when stored rows exceed the reference's norm gate
+    bool odd_rows = false;          // some stored row has an inf / NaN / fp16-overflowing component: only the scan is exact
     size_t q_cap = 0;               // queries
     float *d_queries = nullptr, *h_queries = nullptr;
     // results of the host API: ONE packed block (labels | distances | counts | flags | status) so that a
@@ -159,10 +160,10 @@ struct dawn_index {
     bool bulk_ready = false;
 
     // norm bookkeeping for the certificate: rows [0, norm_checked) have been through the gate scan
-    uint32_t *d_norm_stats = nullptr;  // [0] bad rows, [1] max norm (ordered bits), [2] min norm, [3] pad
+    uint32_t *d_norm_stats = nullptr;  // [0] bad rows, [1] max norm (ordered bits), [2] min norm, [3] odd rows (verify_rows_kernel)
     uint32_t *h_norm_stats = nullptr;  // pinned
     size_t norm_checked = 0;
-    uint64_t bad_rows = 0;
+    uint64_t bad_rows = 0, odd_rows = 0;
     float norm_max = 0.f, norm_min = INFINITY;
 
     // device-side counters: [0] queries returned without a certificate by any finalize launch,
@@ -453,7 +454,7 @@ int flush_staged_async(dawn_index *idx) {
     const int cur = idx->stage_cur;
     CK(idx, cudaMemcpyAsync(idx->d_stage, idx->h_stage, n * kDim * sizeof(float), cudaMemcpyHostToDevice, idx->stream));
     if (idx->scalar == DAWN_SCALAR_I8) CK(idx, launch_ingest_i8(idx->d_stage, arena_i8(idx), at, n, idx->stream));
-    else CK(idx, launch_ingest_f16(idx->d_stage, idx->corpus + at * kDim, n, idx->stream));
+    else CK(idx, launch_ingest_f16(idx->d_stage, idx->corpus + at * kDim, n, idx->stream, idx->corpus32 != nullptr));
     if (idx->corpus32)  // the vectors as given, for the exact f32 re-score
         CK(idx, cudaMemcpyAsync(idx->corpus32 + at * kDim, idx->d_stage, n * kDim * sizeof(float), cudaMemcpyDeviceToDevice, idx->stream));
     CK(idx, cudaMemcpyAsync(idx->labels + at, idx->h_stage_labels, n * sizeof(uint64_t), cudaMemcpyHostToDevice, idx->stream));
@@ -498,6 +499,7 @@ int ensure_norms_checked(dawn_index *idx) {
     CK(idx, cudaMemcpyAsync(idx->h_norm_stats, idx->d_norm_stats, 4 * sizeof(uint32_t), cudaMemcpyDeviceToHost, idx->stream));
     CK(idx, cudaStreamSynchronize(idx->stream));
     idx->bad_rows = idx->h_norm_stats[0];
+    idx->odd_rows = idx->h_norm_stats[3];
     memcpy(&idx->norm_max, &idx->h_norm_stats[1], 4);
     uint32_t inv = ~idx->h_norm_stats[2];
     memcpy(&idx->norm_min, &inv, 4);
@@ -505,7 +507,10 @@ int ensure_norms_checked(dawn_index *idx) {
     return DAWN_OK;
 }
 
+// DAWN_SCALAR_F32 selects on fp16 copies saturated at +-65504: a copy that saturated (or holds inf / NaN) is off by more than
+// any slack, so such an index answers but certifies nothing.
 inline float eps_scale_of(const dawn_index *idx) {
+    if (idx->odd_rows && idx->scalar == DAWN_SCALAR_F32) return INFINITY;
     return idx->norm_max > kRowNormGate ? idx->norm_max / 1.01f * 1.001f : 1.0f;
 }
 
@@ -515,6 +520,7 @@ void reset_norm_stats(dawn_index *idx) {
     cudaStreamSynchronize(idx->stream);
     idx->norm_checked = 0;
     idx->bad_rows = 0;
+    idx->odd_rows = 0;
     idx->norm_max = 0.f;
     idx->norm_min = INFINITY;
 }
@@ -940,6 +946,10 @@ int search_enqueue(dawn_index *idx, SearchWs *ws, const float *d_queries, size_t
     const float store_slack = f32_store ? kF32StoreSlack : 0.0f;
     if (f32_store && kprime < 64) kprime = 64;
     const bool i8_small_on_big = (int64_t)batch >= idx->gemm_small_batch && (int64_t)n >= idx->gemm_small_batch_rows;
+    // A row with an inf or NaN component (or, in an fp16 copy, one at +-65504) breaks the tensor-core paths and the shadow: an
+    // fp16 query component below 2^-25 is 0 there and 0 * inf is NaN, and the shadow stores such a row as zeros.  The scan
+    // multiplies by the f32 query, in the order the oracle does, so it alone answers such an index.
+    if (ws->odd_rows) scan_only = true;
     if (idx->scalar == DAWN_SCALAR_I8 && !scan_only && idx->i8_tensor_min_batch > 0 &&
         ((int64_t)batch >= idx->i8_tensor_min_batch || i8_small_on_big) && n >= 65536 && idx->i8_native)
         return search_i8_native(idx, ws, d_queries, batch, k, kprime, d_labels_out, d_dist_out, d_counts, d_flags, s, d_status_out);
@@ -1099,7 +1109,9 @@ int search_enqueue(dawn_index *idx, SearchWs *ws, const float *d_queries, size_t
         sl.chunk_counter = ws->d_counters + 1 + pass;
         sl.status = ws->d_counters;
         sl.grid = grid;
-        sl.score_floor = limit_score > -INFINITY ? limit_score - 2.0f * (kScanEps + store_slack) - 1e-6f : -INFINITY;
+        // no pushed-down limit: the scan's error grows with |q|, which the host does not know for device-resident queries, so
+        // a floor of limit_score - 2 eps dropped hits of long queries (limit applied afterwards, by the callers)
+        sl.score_floor = -INFINITY;
         EventPair ev;
         bool timed = begin_event(idx, ws, 0, s, &ev);
         CK(idx, launch_scan_topk_f16(sl, s));
@@ -1139,7 +1151,8 @@ int search_enqueue(dawn_index *idx, SearchWs *ws, const float *d_queries, size_t
 }
 
 // Snapshot the searchable state: flush staged adds, run the norm gate over new rows, take the shared corpus lock.
-int snapshot_for_search(dawn_index *idx, std::shared_lock<std::shared_mutex> &rd, size_t *n_rows, float *eps_scale) {
+int snapshot_for_search(dawn_index *idx, std::shared_lock<std::shared_mutex> &rd, size_t *n_rows, float *eps_scale,
+                        bool *odd_rows = nullptr) {
     std::lock_guard<std::mutex> lk(idx->mu);
     int rc = flush_staged(idx);
     if (rc) return rc;
@@ -1149,6 +1162,7 @@ int snapshot_for_search(dawn_index *idx, std::shared_lock<std::shared_mutex> &rd
     if (rc) return rc;
     *n_rows = idx->size;
     *eps_scale = eps_scale_of(idx);
+    if (odd_rows) *odd_rows = idx->odd_rows != 0;
     rd = std::shared_lock<std::shared_mutex>(idx->corpus_mu);
     return DAWN_OK;
 }
@@ -1164,7 +1178,8 @@ int search_batch_host(dawn_index *idx, const float *queries, size_t batch, size_
     std::shared_lock<std::shared_mutex> rd;
     size_t n = 0;
     float eps_scale = 1.0f;
-    rc = snapshot_for_search(idx, rd, &n, &eps_scale);
+    bool odd_rows = false;
+    rc = snapshot_for_search(idx, rd, &n, &eps_scale, &odd_rows);
     if (rc) return rc;
     if (k == 0 || n == 0) {
         for (size_t b = 0; b < batch; b++) counts_out[b] = 0;
@@ -1175,6 +1190,7 @@ int search_batch_host(dawn_index *idx, const float *queries, size_t batch, size_
     if (!ws) return fail(DAWN_ERR_CUDA, "cannot create a search workspace (stream / event creation failed)");
     ws->n_rows = n;
     ws->eps_scale = eps_scale;
+    ws->odd_rows = odd_rows;
     ws->limit_score = (distance_limit == distance_limit && distance_limit < INFINITY) ? (float)(1.0 - (double)distance_limit)
                                                                                       : -INFINITY;
     rc = ensure_query_ws(idx, ws, batch, k);
@@ -1294,7 +1310,8 @@ int bulk_add(dawn_index *idx, const uint64_t *labels, const float *vectors, size
             cudaError_t e = cudaMemcpyAsync(L.d_buf[turn], L.h_buf[turn], cnt * kDim * sizeof(float), cudaMemcpyHostToDevice, L.stream);
             if (e == cudaSuccess)
                 e = idx->scalar == DAWN_SCALAR_I8 ? launch_ingest_i8(L.d_buf[turn], arena_i8(idx), at + r0, cnt, L.stream)
-                                                  : launch_ingest_f16(L.d_buf[turn], idx->corpus + (at + r0) * kDim, cnt, L.stream);
+                                                  : launch_ingest_f16(L.d_buf[turn], idx->corpus + (at + r0) * kDim, cnt, L.stream,
+                                                                      idx->corpus32 != nullptr);
             if (e == cudaSuccess && idx->corpus32)
                 e = cudaMemcpyAsync(idx->corpus32 + (at + r0) * kDim, L.d_buf[turn], cnt * kDim * sizeof(float), cudaMemcpyDeviceToDevice, L.stream);
             if (e == cudaSuccess)
@@ -1574,7 +1591,7 @@ int dawn_index_add_synthetic(dawn_index *idx, uint64_t seed, uint64_t first_row,
     if (idx->scalar == DAWN_SCALAR_I8) CK(idx, launch_synth_i8(arena_i8(idx), at, seed, first_row, n, idx->stream));
     else if (idx->scalar == DAWN_SCALAR_F32) {
         CK(idx, launch_synth_f32(idx->corpus32 + at * kDim, seed, first_row, n, idx->stream));
-        CK(idx, launch_ingest_f16(idx->corpus32 + at * kDim, idx->corpus + at * kDim, n, idx->stream));
+        CK(idx, launch_ingest_f16(idx->corpus32 + at * kDim, idx->corpus + at * kDim, n, idx->stream, true));
     } else CK(idx, launch_synth_f16(idx->corpus + at * kDim, seed, first_row, n, idx->stream));
     CK(idx, launch_iota_labels(idx->labels + at, first_row + 1, n, idx->stream));  // labels = first_row + i + 1
     CK(idx, cudaStreamSynchronize(idx->stream));
@@ -1654,7 +1671,8 @@ int dawn_index_search_device_limit(dawn_index *idx, const float *d_queries, size
     std::shared_lock<std::shared_mutex> rd;
     size_t n = 0;
     float eps_scale = 1.0f;
-    rc = snapshot_for_search(idx, rd, &n, &eps_scale);
+    bool odd_rows = false;
+    rc = snapshot_for_search(idx, rd, &n, &eps_scale, &odd_rows);
     if (rc) return rc;
     std::lock_guard<std::mutex> lk(idx->dev_mu);
     SearchWs *ws = idx->dev_ws;
@@ -1667,6 +1685,7 @@ int dawn_index_search_device_limit(dawn_index *idx, const float *d_queries, size
     const bool limited = distance_limit == distance_limit && distance_limit < INFINITY;
     ws->n_rows = n;
     ws->eps_scale = eps_scale;
+    ws->odd_rows = odd_rows;
     ws->limit_score = limited ? (float)(1.0 - (double)distance_limit) : -INFINITY;
     // the workspace is shared by all device-API searches on this handle: a search enqueued on another
     // stream than the previous one first waits for it
@@ -1898,7 +1917,7 @@ int dawn_index_load(dawn_index *idx, const char *path) {
     slurp(nl, h.size * sizeof(uint64_t));
     if (idx->scalar == DAWN_SCALAR_F32) {
         slurp(n32, payload);
-        if (ok && ce == cudaSuccess && h.size) ce = launch_ingest_f16(n32, nc, (size_t)h.size, idx->stream);  // rebuild the selection copy
+        if (ok && ce == cudaSuccess && h.size) ce = launch_ingest_f16(n32, nc, (size_t)h.size, idx->stream, true);  // rebuild the selection copy
     } else {
         slurp(nc, payload);
     }
@@ -2225,17 +2244,21 @@ __global__ void __launch_bounds__(256) find_label_kernel(const uint64_t *__restr
         if (labels[i] == label) atomicMin(row_out, (uint32_t)i);
 }
 
-// Norm gate over stored rows, one warp per row (vector.rs:181-192 applied to what is actually stored).
+// Norm gate over stored rows, one warp per row (vector.rs:181-192 applied to what is actually stored).  stats[3] counts the odd
+// rows: an fp16 row with an inf / NaN component or one at +-65504 (the saturated copy of an f32 value out of the fp16 range),
+// an int8 row with an infinite scale.  An int8 row whose squared norm overflows f32 (components ~1e30) still gets its finite
+// norm, so the eps scale covers it.
 __global__ void __launch_bounds__(256) verify_rows_kernel(const uint8_t *__restrict__ arena, int scalar, size_t first, size_t n,
                                                           uint32_t *__restrict__ stats) {
     const int lane = threadIdx.x & 31;
     const size_t warp = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const size_t n_warps = ((size_t)gridDim.x * blockDim.x) >> 5;
-    uint32_t bad = 0;
+    uint32_t bad = 0, odd_rows = 0;
     float vmax = 0.f, vmin = __int_as_float(0x7f800000);
     for (size_t r = warp; r < n; r += n_warps) {
         const size_t row = first + r;
-        float acc = 0.f;
+        float acc = 0.f, isf = 0.f, sc = 1.f;
+        bool odd = false;
         if (scalar == 0) {
             const __half *src = reinterpret_cast<const __half *>(arena) + row * kDim;
             const uint4 u = *reinterpret_cast<const uint4 *>(src + lane * 8);
@@ -2247,16 +2270,19 @@ __global__ void __launch_bounds__(256) verify_rows_kernel(const uint8_t *__restr
                 const float2 x = __half22float2(h[j]);
                 acc = fmaf(x.x, x.x, acc);
                 acc = fmaf(x.y, x.y, acc);
+                odd |= !(fabsf(x.x) < 65504.f) || !(fabsf(x.y) < 65504.f);
             }
 #pragma unroll
             for (int j = 0; j < 2; j++) {
                 const float2 x = __half22float2(g[j]);
                 acc = fmaf(x.x, x.x, acc);
                 acc = fmaf(x.y, x.y, acc);
+                odd |= !(fabsf(x.x) < 65504.f) || !(fabsf(x.y) < 65504.f);
             }
         } else {
             const int8_t *src = reinterpret_cast<const int8_t *>(arena + i8_row_offset(row));
-            const float sc = *reinterpret_cast<const float *>(arena + i8_scale_offset(row));
+            sc = *reinterpret_cast<const float *>(arena + i8_scale_offset(row));
+            odd = !(sc < INFINITY);
             const uint2 u = *reinterpret_cast<const uint2 *>(src + lane * 8);
             const uint32_t v = *reinterpret_cast<const uint32_t *>(src + 256 + lane * 4);
             const int8_t *a = reinterpret_cast<const int8_t *>(&u);
@@ -2267,12 +2293,19 @@ __global__ void __launch_bounds__(256) verify_rows_kernel(const uint8_t *__restr
 #pragma unroll
             for (int j = 0; j < 4; j++) isum += (int)b[j] * (int)b[j];
             acc = (float)isum * sc * sc;
+            isf = (float)isum;
         }
 #pragma unroll
-        for (int off = 16; off > 0; off >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, off);
-        const float len = sqrtf(acc);
+        for (int off = 16; off > 0; off >>= 1) {
+            acc += __shfl_xor_sync(0xffffffffu, acc, off);
+            isf += __shfl_xor_sync(0xffffffffu, isf, off);
+        }
+        odd = __any_sync(0xffffffffu, odd);
+        float len = sqrtf(acc);
+        if (!(len < INFINITY) && !odd) len = sqrtf(isf) * sc;  // int8 only: isum * sc * sc overflowed
         const bool finite = len == len && len < __int_as_float(0x7f800000);
         if (!(finite && len > 0.99f && len < 1.01f)) bad++;
+        if (odd) odd_rows++;
         if (finite) {
             vmax = fmaxf(vmax, len);
             vmin = fminf(vmin, len);
@@ -2280,6 +2313,7 @@ __global__ void __launch_bounds__(256) verify_rows_kernel(const uint8_t *__restr
     }
     if (lane == 0) {
         if (bad) atomicAdd(&stats[0], bad);
+        if (odd_rows) atomicAdd(&stats[3], odd_rows);
         atomicMax(&stats[1], __float_as_uint(vmax));      // norms are >= 0: the bit pattern orders like the value
         atomicMax(&stats[2], ~__float_as_uint(vmin));     // min kept inverted so that zero-initialised memory means "none yet"
     }
@@ -2336,8 +2370,9 @@ namespace dawn {
 // Only rows [first, first + n) are written and only they enter their group's maximum: rows below `first` may already be read
 // by searches in flight, so a group that straddles an append keeps its old rows' scale and its new rows get their own.
 // The chunk test takes the largest scale of the chunk, so such a chunk stays rigorous, only looser.
-// Zero rows and rows with inf / NaN (which cannot be a hit of a normalised query) are stored as zeros under the group's scale
-// and are left out of its maximum; a group of nothing but such rows gets scale 1.
+// Zero rows and rows with inf / NaN are stored as zeros under the group's scale and are left out of its maximum; a group of
+// nothing but such rows gets scale 1.  Such a row can be a hit (an inf component scores +-inf), so the searches do not use the
+// shadow while the norm gate counts one (search_enqueue).
 // One block of 8 warps per group, 4 rows per warp.  kappa_bits collects max ||x16 / s - x8|| over the rows with the stored s
 // (<= sqrt(384) / 2 = 9.8 for any s >= absmax / 127, ~5.7-6.3 on real rows): the filter's rigorous bound on a row's own
 // quantisation error is ||q|| * kappa * s_row.

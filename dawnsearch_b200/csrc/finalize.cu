@@ -263,6 +263,7 @@ finalize_kernel(const __half *__restrict__ corpus, const float *__restrict__ que
     FIN_TRACE(5);
     Cand mine = empty_cand();
     float my_scan = __int_as_float(0x7f800000);  // scan score of this candidate (+inf for an empty slot)
+    bool dropped = false;                        // a candidate whose exact score is NaN: not a result, yet it held a slot
     if (tid < kp) {
         mine = sm.s[tid];
         my_scan = mine.row != kNoRow ? mine.score : __int_as_float(0x7f800000);
@@ -315,6 +316,10 @@ finalize_kernel(const __half *__restrict__ corpus, const float *__restrict__ que
                     atomicMax(&stats[2], __float_as_uint(err));
             }
             mine.score = __fsub_rn(1.0f, acc);  // distance, vector.rs:133
+            if (acc != acc) {
+                dropped = true;
+                mine.row = kNoRow;
+            }
         }
     }
     __syncthreads();  // every read of the merged list is done before it is overwritten with distances
@@ -338,6 +343,7 @@ finalize_kernel(const __half *__restrict__ corpus, const float *__restrict__ que
         if (tid == 0) sm.q_norm2 = a;
     }
     const int n_valid = __syncthreads_count(valid ? 1 : 0);
+    const int n_held = __syncthreads_count(valid || dropped ? 1 : 0);  // candidates the lists held
 
     // ---- final order: distance asc, label asc, row asc (rank counting over <= 128 entries).
     // Ordering on the emitted f32 distance (not the score) makes the output self-consistent
@@ -354,7 +360,7 @@ finalize_kernel(const __half *__restrict__ corpus, const float *__restrict__ que
     if (tid == 0) {
         counts_out[qi] = (uint32_t)min(k, n_valid);
         bool certified = true;
-        if (n_valid == kp) {
+        if (n_held == kp) {
             // A row outside the candidate set has scan score <= scan_min, hence exact score
             // <= scan_min + eps and distance >= 1 - (scan_min + eps); it cannot displace or tie
             // the k-th result if that bound is strictly above the k-th distance.
@@ -365,7 +371,7 @@ finalize_kernel(const __half *__restrict__ corpus, const float *__restrict__ que
             for (int w = 1; w < (kp + 31) / 32; w++) wmin = min(wmin, sm.warp_min[w]);
             const float scan_min = ordered_to_float(wmin);  // weakest kept candidate (lists need not be sorted)
             const float bound = __fsub_rn(1.0f, __fadd_rn(scan_min, e));
-            certified = bound > sm.kth_dist;
+            certified = n_valid >= k && bound > sm.kth_dist;  // NaN drops can leave fewer than k: rows outside may be missing
         }
         if (overflow && overflow[qi]) certified = false;  // candidates were lost: cannot certify
         flags_out[qi] = certified ? 1u : 0u;

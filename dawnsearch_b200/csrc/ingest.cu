@@ -15,11 +15,19 @@ namespace dawn {
 
 namespace {
 
+// saturate: the selection copy of DAWN_SCALAR_F32 rows keeps every non-NaN value at most +-65504, so that a value out of the
+// fp16 range still ranks its row near where it belongs (an inf copy would give inf - inf = NaN and drop the row).
+__device__ __forceinline__ float sat_f16(float v) { return v < -65504.f ? -65504.f : v > 65504.f ? 65504.f : v; }
+
 __global__ void __launch_bounds__(256) ingest_f16_kernel(const float4 *__restrict__ src,
-                                                         uint4 *__restrict__ dst, size_t n_vec8) {
+                                                         uint4 *__restrict__ dst, size_t n_vec8, bool saturate) {
     size_t stride = (size_t)gridDim.x * blockDim.x;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_vec8; i += stride) {
         float4 a = src[2 * i], b = src[2 * i + 1];
+        if (saturate) {
+            a = make_float4(sat_f16(a.x), sat_f16(a.y), sat_f16(a.z), sat_f16(a.w));
+            b = make_float4(sat_f16(b.x), sat_f16(b.y), sat_f16(b.z), sat_f16(b.w));
+        }
         __half2 h0 = __floats2half2_rn(a.x, a.y), h1 = __floats2half2_rn(a.z, a.w);
         __half2 h2 = __floats2half2_rn(b.x, b.y), h3 = __floats2half2_rn(b.z, b.w);
         uint4 o;
@@ -121,7 +129,7 @@ __device__ __forceinline__ void quantize_row_i8(const float (&x)[12], uint8_t *a
 #pragma unroll
     for (int j = 0; j < 12; j++) {
         float q = roundf(__fdiv_rn(x[j], scale));
-        q = fminf(127.f, fmaxf(-127.f, q));
+        q = q == q ? fminf(127.f, fmaxf(-127.f, q)) : 0.f;  // a NaN quotient (NaN, or inf / inf) stores 0, as Rust's `as` does
         qv[j] = (int8_t)q;
     }
     uint8_t *row = arena + i8_row_offset(dst_row);
@@ -212,13 +220,13 @@ cudaError_t launch_gather_f32_i8(const uint8_t *arena, const uint32_t *rows, siz
     return cudaGetLastError();
 }
 
-cudaError_t launch_ingest_f16(const float *src_f32, __half *dst, size_t n_rows, cudaStream_t s) {
+cudaError_t launch_ingest_f16(const float *src_f32, __half *dst, size_t n_rows, cudaStream_t s, bool saturate) {
     if (n_rows == 0) return cudaSuccess;
     size_t n_vec8 = n_rows * (kDim / 8);
     size_t blocks = (n_vec8 + 255) / 256;
     if (blocks > 148 * 16) blocks = 148 * 16;
     ingest_f16_kernel<<<(unsigned)blocks, 256, 0, s>>>(reinterpret_cast<const float4 *>(src_f32),
-                                                      reinterpret_cast<uint4 *>(dst), n_vec8);
+                                                      reinterpret_cast<uint4 *>(dst), n_vec8, saturate);
     return cudaGetLastError();
 }
 

@@ -55,6 +55,7 @@ typedef struct {
 } topk_t;
 
 static void topk_push(topk_t *t, cand_t c) {
+    if (c.score != c.score) return; /* a NaN score is not a result (dawn_oracle.c) */
     int (*better)(const cand_t *, const cand_t *) = t->final ? final_better : cand_better;
     if (t->len == t->k) {
         if (!better(&c, &t->v[t->len - 1])) return;

@@ -211,6 +211,7 @@ void dawn_oracle_store_i8(const float *rows, size_t n, int8_t *out, float *scale
         scales[r] = scale;
         for (int i = 0; i < EM; i++) {
             float q = roundf(x[i] / scale);
+            if (q != q) q = 0.0f; /* a NaN quotient (NaN or inf / inf) stores 0, as Rust's `as` does */
             if (q > 127.0f) q = 127.0f;
             if (q < -127.0f) q = -127.0f;
             out[r * EM + i] = (int8_t)q;
@@ -282,8 +283,10 @@ typedef struct {
     size_t k, len;
 } topk_t;
 
+/* A row whose exact score is NaN is not a result: NaN has no place in the total order, and keeping it
+ * would make the output depend on row order.  +-inf scores are ordered (distance -inf is best). */
 static void topk_push(topk_t *t, cand_t c) {
-    if (t->k == 0) return;
+    if (t->k == 0 || c.score != c.score) return;
     if (t->len == t->k) {
         if (!cand_better(&c, &t->v[t->len - 1])) return;
         t->len--;

@@ -415,15 +415,17 @@ def np_scores_seq(stored_f32: np.ndarray, query: np.ndarray) -> np.ndarray:
 
 
 def np_search(stored_f32: np.ndarray, labels, query, k: int, row_scale=None):
-    """Exact top-k by (distance asc, label asc, row asc); distance = 1 - score (f32)."""
+    """Exact top-k by (distance asc, label asc, row asc); distance = 1 - score (f32).  Rows whose score is NaN
+    are not results, so the count is min(k, rows with a non-NaN score)."""
     n = stored_f32.shape[0]
-    scores = np_scores_seq(stored_f32, query)
-    if row_scale is not None:
-        scores = (np.asarray(row_scale, dtype=np.float32) * scores).astype(np.float32)
+    with np.errstate(invalid="ignore", over="ignore"):
+        scores = np_scores_seq(stored_f32, query)
+        if row_scale is not None:
+            scores = (np.asarray(row_scale, dtype=np.float32) * scores).astype(np.float32)
     dist = (np.float32(1.0) - scores).astype(np.float32)
     lab = np.arange(1, n + 1, dtype=np.uint64) if labels is None else np.asarray(labels, dtype=np.uint64)
     order = np.lexsort((np.arange(n), lab, dist))
-    order = order[: min(k, n)]
+    order = order[~np.isnan(dist[order])][:k]
     return lab[order].copy(), dist[order].copy()
 
 
@@ -470,13 +472,15 @@ def np_clustered_rows_f32(seed: int, first_row: int, n: int, centers: int = 1024
 
 def np_store_i8(rows: np.ndarray):
     """numpy twin of dawn_oracle_store_i8: scale = absmax/127 (f32 division), q = roundf(x/scale) (half away
-    from zero, the reference's rounding at src/search/vector.rs:30-32), clamped to +-127."""
+    from zero, the reference's rounding at src/search/vector.rs:30-32), clamped to +-127; a NaN quotient (a NaN component,
+    or an inf one over an inf scale) stores 0, as Rust's `as` does.  NaN components are left out of absmax."""
     rows = np.ascontiguousarray(rows, dtype=np.float32).reshape(-1, EM_LEN)
-    amax = np.abs(rows).max(axis=1).astype(np.float32)
+    amax = np.abs(np.where(np.isnan(rows), np.float32(0), rows)).max(axis=1).astype(np.float32)
     scale = np.where(amax > 0, (amax / np.float32(127.0)).astype(np.float32), np.float32(1.0)).astype(np.float32)
-    t64 = (rows / scale[:, None]).astype(np.float32).astype(np.float64)  # the f32 quotient; +-0.5 is exact in f64
-    q = np.where(t64 >= 0, np.floor(t64 + 0.5), np.ceil(t64 - 0.5))
-    q = np.clip(q, -127, 127)
+    with np.errstate(invalid="ignore"):
+        t64 = (rows / scale[:, None]).astype(np.float32).astype(np.float64)  # the f32 quotient; +-0.5 is exact in f64
+        q = np.where(t64 >= 0, np.floor(t64 + 0.5), np.ceil(t64 - 0.5))
+    q = np.where(np.isnan(q), 0, np.clip(q, -127, 127))
     return q.astype(np.int8), scale
 
 
