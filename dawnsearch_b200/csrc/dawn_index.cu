@@ -2116,9 +2116,9 @@ int dawn_merge_results_device(int device, const uint64_t *d_labels, const float 
                               uint32_t *d_counts_out, void *stream) {
     if (!d_labels || !d_distances || !d_counts || !d_labels_out || !d_distances_out || !d_counts_out)
         return fail(DAWN_ERR_INVALID, "null device pointer");
-    if (k == 0 || k > DAWN_MAX_K || n_lists == 0 || n_lists * k > 1024)
-        return fail(DAWN_ERR_INVALID, "merge shape out of range (n_lists=%zu k=%zu; n_lists*k must be <= 1024)",
-                    n_lists, k);
+    if (k == 0 || k > DAWN_MAX_K || n_lists == 0 || n_lists > 64 || n_lists * k > 1024)
+        return fail(DAWN_ERR_INVALID,
+                    "merge shape out of range (n_lists=%zu k=%zu; n_lists must be <= 64 and n_lists*k <= 1024)", n_lists, k);
     if (batch == 0) return DAWN_OK;
     cudaError_t e = cudaSetDevice(device);
     if (e == cudaSuccess)
@@ -2156,7 +2156,8 @@ __global__ void __launch_bounds__(1024) merge_results_kernel(
     // list l's arrays start l * stride bytes after the base pointers (dense arrays or one packed
     // block per shard as it arrives from the all-gather)
     if (tid < n_lists)
-        s_cnt[tid] = min((int)reinterpret_cast<const uint32_t *>(reinterpret_cast<const char *>(counts) + tid * stride_c)[qi], k);
+        s_cnt[tid] = (int)min(reinterpret_cast<const uint32_t *>(reinterpret_cast<const char *>(counts) + tid * stride_c)[qi],
+                              (uint32_t)k);  // unsigned: a count past INT_MAX is still clamped to k
     if (tid < total) {
         const int l = tid / k, p = tid % k;
         s_lab[tid] = reinterpret_cast<const uint64_t *>(reinterpret_cast<const char *>(labels) + l * stride_l)[(size_t)qi * k + p];
@@ -2327,7 +2328,6 @@ __global__ void __launch_bounds__(256) iota_labels_kernel(uint64_t *__restrict__
 cudaError_t launch_merge_results(const uint64_t *labels, const float *dist, const uint32_t *counts, int n_lists,
                                  size_t list_stride_bytes, int batch, int k, uint64_t *labels_out, float *dist_out,
                                  uint32_t *counts_out, cudaStream_t s) {
-    if (n_lists > 64) return cudaErrorInvalidValue;
     size_t sl = list_stride_bytes, sd = list_stride_bytes, sc = list_stride_bytes;
     if (list_stride_bytes == 0) {  // dense [n_lists][batch][k] arrays
         sl = (size_t)batch * k * sizeof(uint64_t);

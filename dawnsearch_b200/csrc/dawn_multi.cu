@@ -12,8 +12,10 @@
 // (The one-process-per-GPU variant of the same exchange under torch.distributed is dawnsearch_b200/sharded.py.)
 //
 // Exactness: shards return bit-exact distances, the merge orders by (distance, label), so the
-// answer equals a single index holding everything.  Queries a shard could not certify are re-run
-// on that shard through the exact scan before the merge.
+// answer equals a single index holding everything as long as every label is stored once (a label
+// stored on two shards at the same distance comes back once: include/dawn_index.h,
+// dawn_merge_results_device).  Queries a shard could not certify are re-run on that shard through
+// the exact scan before the merge.
 #include <atomic>
 #include <condition_variable>
 #include <cstdlib>

@@ -7,7 +7,8 @@ one NVSwitch box the same shape becomes: local exact top-k on every GPU (libdawn
 ONE all-gather of a packed block of k (label, distance) pairs per query over NCCL/NVLink ->
 device-side merge (dawn_merge_results_device).  Because every shard returns bit-exact
 distances and the order is defined on (distance, label), the merged result is bit-identical
-to a single index holding the whole corpus.
+to a single index holding the whole corpus (with every label stored once: a label two shards
+hold at the same distance comes back once, see dawn_merge_results_device).
 
 torch is plumbing here (device buffers, streams, torch.distributed); all compute is in
 libdawn_b200.so.

@@ -156,7 +156,12 @@ int dawn_index_search_device_limit(dawn_index *idx, const float *d_queries, size
  * src/search/search_service.rs:247-268).  List l's three arrays start l*list_stride_bytes
  * after the three base pointers, so one packed block per shard (as it lands from a single
  * all-gather) can be merged in place; list_stride_bytes == 0 means three dense arrays
- * [n_lists][batch][k] / [n_lists][batch].  n_lists*k <= 1024. */
+ * [n_lists][batch][k] / [n_lists][batch].  n_lists <= 64 and n_lists*k <= 1024, else DAWN_ERR_INVALID.
+ * The rule: each list's first min(count, k) entries; an entry whose (distance, label) also occurs in a list
+ * with a smaller index is dropped (a page stored on two shards); the rest ordered by (distance, label, list
+ * index); the first k kept.  With every label stored once this is one index holding every list's rows; a
+ * label stored on several shards at the same distance is returned as often as the lowest-index shard holding
+ * it returns it.  Nothing past counts_out[b] is written. */
 int dawn_merge_results_device(int device, const uint64_t *d_labels, const float *d_distances,
                               const uint32_t *d_counts, size_t n_lists, size_t list_stride_bytes,
                               size_t batch, size_t k, uint64_t *d_labels_out, float *d_distances_out,
