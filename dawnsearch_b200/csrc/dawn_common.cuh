@@ -275,5 +275,8 @@ struct RemoveMove {
 };
 // move: copy every row, scale and label of donors[i] into holes[i].
 cudaError_t launch_remove_move(const RemoveMove &p, cudaStream_t s);
+// Load into another shard count (persist.cuh, fill_rows): rows [src_first, src_first + n) of the blocked int8 blocks staged
+// at `src` move, each with its scale, to rows [dst_first, dst_first + n) of the blocked arena `dst`.
+cudaError_t launch_reblock_i8(const uint8_t *src, size_t src_first, uint8_t *dst, size_t dst_first, size_t n, cudaStream_t s);
 
 }  // namespace dawn

@@ -20,6 +20,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <chrono>
+#include <functional>
 #include <condition_variable>
 #include <mutex>
 #include <new>
@@ -28,8 +29,14 @@
 #include <thread>
 #include <vector>
 
+#include <errno.h>
+#include <fcntl.h>
+#include <sys/stat.h>
+#include <unistd.h>
+
 #include "../../include/dawn_index.h"
 #include "dawn_common.cuh"
+#include "persist.cuh"
 
 using namespace dawn;
 
@@ -1767,6 +1774,7 @@ int dawn_index_verify(dawn_index *idx, size_t *bad_rows_out, float *min_norm_out
 }
 
 // ---- save / load: header, labels, stored rows (raw device layout) -------------------------
+// The section writer and the two-phase fill live in namespace dawn below (persist.cuh); dawn_multi_save / _load use them too.
 struct SaveHeader {
     char magic[8];  // "DAWNB200"
     uint32_t version, scalar, dims, reserved;
@@ -1778,65 +1786,20 @@ int dawn_index_save(dawn_index *idx, const char *path) {
     if (rc) return rc;
     if (!path) return fail(DAWN_ERR_INVALID, "path is null");
     std::lock_guard<std::mutex> lk(idx->mu);
-    rc = flush_staged(idx);
+    uint64_t n = 0;
+    rc = section_prepare(idx, true, &n);
     if (rc) return rc;
-    const size_t n = idx->size;
-    if (idx->scalar == DAWN_SCALAR_I8 && n % kI8BlockRows) {
-        // the last 8-row block is partly unused: zero its unused rows and scales so the file is deterministic
-        const size_t blk_end = (n + kI8BlockRows - 1) / kI8BlockRows * kI8BlockRows;
-        CK(idx, cudaMemsetAsync(arena_i8(idx) + i8_row_offset(n), 0, (blk_end - n) * kDim, idx->stream));
-        CK(idx, cudaMemsetAsync(arena_i8(idx) + i8_scale_offset(n), 0, (blk_end - n) * 4, idx->stream));
-    }
     std::string tmp = std::string(path) + ".tmp";
-    FILE *f = fopen(tmp.c_str(), "wb");
-    if (!f) return fail(DAWN_ERR_IO, "cannot open %s for writing", tmp.c_str());
+    int fd = open(tmp.c_str(), O_WRONLY | O_CREAT | O_TRUNC | O_CLOEXEC, 0666);
+    if (fd < 0) return fail(DAWN_ERR_IO, "cannot open %s for writing", tmp.c_str());
     SaveHeader h{};
     memcpy(h.magic, "DAWNB200", 8);
     h.version = 1;
     h.scalar = (uint32_t)idx->scalar;
     h.dims = kDim;
     h.size = n;
-    bool ok = fwrite(&h, sizeof h, 1, f) == 1;
-    // stream device memory out through the two pinned staging buffers: the D2H of slice i+1 runs while
-    // slice i is written to the file
-    const size_t buf_bytes = kStageRowsHost * kDim * sizeof(float);
-    auto dump = [&](const void *dptr, size_t bytes) -> int {
-        size_t off = 0;
-        int cur = 0;
-        size_t in_flight = 0;
-        if (bytes) {
-            in_flight = bytes < buf_bytes ? bytes : buf_bytes;
-            CK(idx, cudaMemcpyAsync(idx->h_stage_buf[0], dptr, in_flight, cudaMemcpyDeviceToHost, idx->stream));
-        }
-        while (ok && off < bytes) {
-            CK(idx, cudaStreamSynchronize(idx->stream));
-            const size_t have = in_flight;
-            const size_t next_off = off + have;
-            if (next_off < bytes) {
-                in_flight = bytes - next_off < buf_bytes ? bytes - next_off : buf_bytes;
-                CK(idx, cudaMemcpyAsync(idx->h_stage_buf[cur ^ 1], (const char *)dptr + next_off, in_flight, cudaMemcpyDeviceToHost,
-                                        idx->stream));
-            }
-            ok = fwrite(idx->h_stage_buf[cur], 1, have, f) == have;
-            off = next_off;
-            cur ^= 1;
-        }
-        CK(idx, cudaStreamSynchronize(idx->stream));
-        return DAWN_OK;
-    };
-    rc = dump(idx->labels, n * sizeof(uint64_t));
-    if (rc == DAWN_OK)  // F32 storage persists the vectors as given; the fp16 selection copy is rebuilt on load
-        rc = idx->scalar == DAWN_SCALAR_F32 ? dump(idx->corpus32, n * (size_t)kDim * sizeof(float)) : dump(idx->corpus, arena_bytes(idx, n));
-    ok = (fclose(f) == 0) && ok;
-    if (rc != DAWN_OK || !ok) {
-        remove(tmp.c_str());
-        return rc != DAWN_OK ? rc : fail(DAWN_ERR_IO, "short write to %s", tmp.c_str());
-    }
-    if (rename(tmp.c_str(), path) != 0) {
-        remove(tmp.c_str());
-        return fail(DAWN_ERR_IO, "cannot rename %s to %s", tmp.c_str(), path);
-    }
-    return DAWN_OK;
+    rc = pwrite_all(fd, &h, sizeof h, 0) ? section_write(idx, fd, sizeof h, n) : fail(DAWN_ERR_IO, "short write to %s", tmp.c_str());
+    return finish_file(fd, tmp.c_str(), path, rc);
 }
 
 // Loads into a FRESH arena and swaps it in only when the whole file has arrived, so any failure
@@ -1849,99 +1812,262 @@ int dawn_index_load(dawn_index *idx, const char *path) {
     std::lock_guard<std::mutex> lk(idx->mu);
     rc = flush_staged(idx);  // staged adds belong to the old contents; they must not leak into the loaded ones
     if (rc) return rc;
-    FILE *f = fopen(path, "rb");
-    if (!f) return fail(DAWN_ERR_IO, "cannot open %s", path);
+    int fd = open(path, O_RDONLY | O_CLOEXEC);
+    if (fd < 0) return fail(DAWN_ERR_IO, "cannot open %s", path);
     SaveHeader h{};
-    if (fread(&h, sizeof h, 1, f) != 1 || memcmp(h.magic, "DAWNB200", 8) != 0 || h.version != 1 ||
+    if (!pread_all(fd, &h, sizeof h, 0) || memcmp(h.magic, "DAWNB200", 8) != 0 || h.version != 1 ||
         h.scalar != (uint32_t)idx->scalar || h.dims != kDim) {
-        fclose(f);
+        close(fd);
         return fail(DAWN_ERR_IO, "%s is not a libdawn_b200 index file with this index's storage type", path);
     }
-    fseek(f, 0, SEEK_END);
-    long long flen = ftell(f);
-    const size_t payload = idx->scalar == DAWN_SCALAR_F32 ? (size_t)h.size * kDim * sizeof(float) : arena_bytes(idx, h.size);
-    long long want = (long long)sizeof h + (long long)h.size * 8 + (long long)payload;
+    struct stat st;
+    const long long flen = fstat(fd, &st) == 0 ? (long long)st.st_size : -1;
+    const long long want = h.size > (1ull << 40) ? -1
+                                                : (long long)(sizeof h + h.size * 8 + section_payload_bytes(h.scalar, h.size));
     if (flen != want) {
-        fclose(f);
+        close(fd);
         return fail(DAWN_ERR_IO, "%s is truncated (%lld bytes, expected %lld)", path, flen, want);
     }
-    fseek(f, sizeof h, SEEK_SET);
     if (h.size > 0xFFFFFFF0ull) {
-        fclose(f);
+        close(fd);
         return fail(DAWN_ERR_INVALID, "%s holds more than 2^32 rows", path);
     }
-    size_t rows_alloc = h.size > idx->capacity ? (size_t)h.size : idx->capacity.load();
-    __half *nc = nullptr;
-    uint64_t *nl = nullptr;
-    float *n32 = nullptr;
+    const SectionRef sec{sizeof h, h.size};
+    Fill f;
+    rc = fill_rows(idx, fd, path, &sec, 1, 0, h.size, true, &f);
+    close(fd);
+    if (rc) return rc;
+    fill_commit(idx, &f);
+    return DAWN_OK;
+}
+
+}  // extern "C"
+
+namespace dawn {
+
+bool pwrite_all(int fd, const void *buf, size_t n, uint64_t off) {
+    const char *p = static_cast<const char *>(buf);
+    while (n) {
+        const ssize_t w = pwrite(fd, p, n, (off_t)off);
+        if (w < 0 && errno == EINTR) continue;
+        if (w <= 0) return false;
+        p += w;
+        n -= (size_t)w;
+        off += (uint64_t)w;
+    }
+    return true;
+}
+
+bool pread_all(int fd, void *buf, size_t n, uint64_t off) {
+    char *p = static_cast<char *>(buf);
+    while (n) {
+        const ssize_t r = pread(fd, p, n, (off_t)off);
+        if (r < 0 && errno == EINTR) continue;
+        if (r <= 0) return false;
+        p += r;
+        n -= (size_t)r;
+        off += (uint64_t)r;
+    }
+    return true;
+}
+
+int finish_file(int fd, const char *tmp, const char *path, int rc) {
+    const bool closed = close(fd) == 0;
+    if (rc == DAWN_OK && !closed) rc = fail(DAWN_ERR_IO, "short write to %s", tmp);
+    if (rc != DAWN_OK) {
+        remove(tmp);
+        return rc;
+    }
+    if (rename(tmp, path) != 0) {
+        remove(tmp);
+        return fail(DAWN_ERR_IO, "cannot rename %s to %s", tmp, path);
+    }
+    return DAWN_OK;
+}
+
+uint64_t section_payload_bytes(uint32_t scalar, uint64_t rows) {
+    if (scalar == DAWN_SCALAR_I8) return i8_arena_bytes(rows);
+    return rows * (uint64_t)kDim * (scalar == DAWN_SCALAR_F32 ? sizeof(float) : sizeof(__half));
+}
+
+int section_prepare(dawn_index *idx, bool caller_holds_mu, uint64_t *rows_out) {
+    std::unique_lock<std::mutex> lk(idx->mu, std::defer_lock);
+    if (!caller_holds_mu) lk.lock();
+    int rc = flush_staged(idx);
+    if (rc) return rc;
+    const size_t n = idx->size;
+    if (idx->scalar == DAWN_SCALAR_I8 && n % kI8BlockRows) {
+        // the last 8-row block is partly unused: zero its unused rows and scales so the file is deterministic
+        const size_t blk_end = (n + kI8BlockRows - 1) / kI8BlockRows * kI8BlockRows;
+        CK(idx, cudaMemsetAsync(arena_i8(idx) + i8_row_offset(n), 0, (blk_end - n) * kDim, idx->stream));
+        CK(idx, cudaMemsetAsync(arena_i8(idx) + i8_scale_offset(n), 0, (blk_end - n) * 4, idx->stream));
+        CK(idx, cudaStreamSynchronize(idx->stream));
+    }
+    *rows_out = n;
+    return DAWN_OK;
+}
+
+int section_write(dawn_index *idx, int fd, uint64_t off, uint64_t rows) {
+    std::shared_lock<std::shared_mutex> rd(idx->corpus_mu);
+    const size_t buf_bytes = kStageRowsHost * kDim * sizeof(float);
+    bool ok = true;
+    // stream device memory out through the two pinned staging buffers: the D2H of slice i+1 runs while
+    // slice i is written to the file
+    auto dump = [&](const void *dptr, size_t bytes, uint64_t at) -> int {
+        size_t done = 0;
+        int cur = 0;
+        size_t in_flight = 0;
+        if (bytes) {
+            in_flight = bytes < buf_bytes ? bytes : buf_bytes;
+            CK(idx, cudaMemcpyAsync(idx->h_stage_buf[0], dptr, in_flight, cudaMemcpyDeviceToHost, idx->stream));
+        }
+        while (ok && done < bytes) {
+            CK(idx, cudaStreamSynchronize(idx->stream));
+            const size_t have = in_flight;
+            const size_t next = done + have;
+            if (next < bytes) {
+                in_flight = bytes - next < buf_bytes ? bytes - next : buf_bytes;
+                CK(idx, cudaMemcpyAsync(idx->h_stage_buf[cur ^ 1], (const char *)dptr + next, in_flight, cudaMemcpyDeviceToHost,
+                                        idx->stream));
+            }
+            ok = pwrite_all(fd, idx->h_stage_buf[cur], have, at + done);
+            done = next;
+            cur ^= 1;
+        }
+        CK(idx, cudaStreamSynchronize(idx->stream));
+        return DAWN_OK;
+    };
+    int rc = dump(idx->labels, rows * sizeof(uint64_t), off);
+    if (rc == DAWN_OK)  // F32 storage persists the vectors as given; the fp16 selection copy is rebuilt on load
+        rc = dump(idx->scalar == DAWN_SCALAR_F32 ? (const void *)idx->corpus32 : (const void *)idx->corpus,
+                  section_payload_bytes((uint32_t)idx->scalar, rows), off + rows * sizeof(uint64_t));
+    if (rc != DAWN_OK) return rc;
+    return ok ? DAWN_OK : fail(DAWN_ERR_IO, "short write: %s", strerror(errno));
+}
+
+int fill_rows(dawn_index *idx, int fd, const char *path, const SectionRef *secs, size_t n_secs, uint64_t first, uint64_t n,
+              bool may_fill_in_place, Fill *f) {
+    *f = Fill{};
+    f->rows = n;
     // An EMPTY index with room (the start-up case: reserve, then load) is filled in place -- nothing can be lost, and a
     // second arena next to a pre-reserved 100M-row one would not fit.  Otherwise: fresh arena, swap on success.
-    const bool in_place = idx->size == 0 && idx->phys >= (size_t)h.size && idx->phys > 0;
-    if (in_place) {
+    f->in_place = may_fill_in_place && idx->size == 0 && idx->phys >= n && idx->phys > 0;
+    const size_t want_rows = n > idx->capacity ? (size_t)n : idx->capacity.load();
+    __half *nc = nullptr;
+    if (f->in_place) {
         std::unique_lock<std::shared_mutex> wr(idx->corpus_mu);  // no search may be reading the (empty) arena's pointers
         wait_device_searches(idx);
         nc = idx->corpus;
-        nl = idx->labels;
-        n32 = idx->corpus32;
-        rows_alloc = idx->phys;
-    } else if (rows_alloc > 0) {
-        rc = alloc_arena(idx, rows_alloc, &nc, &nl, &n32);
+        f->labels = idx->labels;
+        f->corpus32 = idx->corpus32;
+        f->rows_alloc = idx->phys;
+    } else if (want_rows > 0) {
+        int rc = alloc_arena(idx, want_rows, &nc, &f->labels, &f->corpus32);
         if (rc) {
-            fclose(f);
+            *f = Fill{};
             return rc;
         }
+        f->rows_alloc = want_rows;
     }
+    f->corpus = nc;
+    cudaStream_t s = idx->stream;
     const size_t buf_bytes = kStageRowsHost * kDim * sizeof(float);
     bool ok = true;
     cudaError_t ce = cudaSuccess;
-    // double-buffered: the file read of slice i+1 overlaps the H2D of slice i
-    auto slurp = [&](void *dptr, size_t bytes) {
-        size_t off = 0;
+    bool busy[2] = {false, false};
+    // File bytes [off, off + bytes) in slices of at most `slice` bytes through the two pinned staging buffers; `sink` enqueues
+    // the device work of one slice on s.  The read of slice i+1 overlaps the copy of slice i.
+    auto stream_in = [&](uint64_t off, uint64_t bytes, size_t slice, const std::function<cudaError_t(int, uint64_t, size_t)> &sink) {
+        uint64_t done = 0;
         int cur = 0;
-        while (ok && ce == cudaSuccess && off < bytes) {
-            const size_t take = bytes - off < buf_bytes ? bytes - off : buf_bytes;
-            if (idx->stage_busy[cur]) {
+        while (ok && ce == cudaSuccess && done < bytes) {
+            const size_t take = bytes - done < slice ? (size_t)(bytes - done) : slice;
+            if (busy[cur]) {
                 ce = cudaEventSynchronize(idx->stage_done[cur]);
-                idx->stage_busy[cur] = false;
+                busy[cur] = false;
                 if (ce != cudaSuccess) break;
             }
-            ok = fread(idx->h_stage_buf[cur], 1, take, f) == take;
+            ok = pread_all(fd, idx->h_stage_buf[cur], take, off + done);
             if (!ok) break;
-            ce = cudaMemcpyAsync((char *)dptr + off, idx->h_stage_buf[cur], take, cudaMemcpyHostToDevice, idx->stream);
-            if (ce == cudaSuccess) ce = cudaEventRecord(idx->stage_done[cur], idx->stream);
-            idx->stage_busy[cur] = true;
-            off += take;
+            ce = sink(cur, done, take);
+            if (ce == cudaSuccess) ce = cudaEventRecord(idx->stage_done[cur], s);
+            busy[cur] = true;
+            done += take;
             cur ^= 1;
         }
     };
-    slurp(nl, h.size * sizeof(uint64_t));
-    if (idx->scalar == DAWN_SCALAR_F32) {
-        slurp(n32, payload);
-        if (ok && ce == cudaSuccess && h.size) ce = launch_ingest_f16(n32, nc, (size_t)h.size, idx->stream, true);  // rebuild the selection copy
-    } else {
-        slurp(nc, payload);
+    auto raw = [&](void *to) {
+        return [&, to](int cur, uint64_t done, size_t take) {
+            return cudaMemcpyAsync((char *)to + done, idx->h_stage_buf[cur], take, cudaMemcpyHostToDevice, s);
+        };
+    };
+    uint8_t *arena = reinterpret_cast<uint8_t *>(nc);
+    uint64_t base = 0, dst = 0;  // first row of section i in the concatenation; next row of this fill
+    for (size_t i = 0; i < n_secs && dst < n && ok && ce == cudaSuccess; i++) {
+        const uint64_t s0 = base, s1 = base + secs[i].rows;
+        base = s1;
+        if (first + dst >= s1) continue;
+        const uint64_t lo = first + dst - s0, hi = (first + n < s1 ? first + n : s1) - s0, cnt = hi - lo;
+        const uint64_t rows_at = secs[i].off + secs[i].rows * sizeof(uint64_t);
+        stream_in(secs[i].off + lo * sizeof(uint64_t), cnt * sizeof(uint64_t), buf_bytes, raw(f->labels + dst));
+        if (idx->scalar == DAWN_SCALAR_F32) {
+            stream_in(rows_at + lo * kDim * sizeof(float), cnt * kDim * sizeof(float), buf_bytes, raw(f->corpus32 + dst * kDim));
+        } else if (idx->scalar == DAWN_SCALAR_F16) {
+            stream_in(rows_at + lo * kRowBytesF16, cnt * kRowBytesF16, buf_bytes, raw(arena + dst * kRowBytesF16));
+        } else if (lo % kI8BlockRows == 0 && dst % kI8BlockRows == 0) {  // whole blocks on both sides
+            stream_in(rows_at + lo / kI8BlockRows * kI8BlockBytes, i8_arena_bytes(cnt), buf_bytes,
+                      raw(arena + dst / kI8BlockRows * kI8BlockBytes));
+        } else {
+            // the source blocks holding rows [lo, hi) are staged on the device and every row moves with its scale into
+            // the destination's blocked layout
+            const uint64_t b0 = lo / kI8BlockRows, b1 = (hi + kI8BlockRows - 1) / kI8BlockRows;
+            const size_t slice = buf_bytes / kI8BlockBytes * kI8BlockBytes;
+            const uint64_t dst0 = dst;
+            stream_in(rows_at + b0 * kI8BlockBytes, (b1 - b0) * kI8BlockBytes, slice, [&](int cur, uint64_t done, size_t take) {
+                cudaError_t e = cudaMemcpyAsync(idx->d_stage_buf[cur], idx->h_stage_buf[cur], take, cudaMemcpyHostToDevice, s);
+                const uint64_t row0 = (b0 + done / kI8BlockBytes) * kI8BlockRows;  // first source row of the slice
+                const uint64_t r0 = lo > row0 ? lo : row0;
+                const uint64_t r1 = hi < row0 + take / kI8BlockBytes * kI8BlockRows ? hi : row0 + take / kI8BlockBytes * kI8BlockRows;
+                if (e == cudaSuccess)
+                    e = launch_reblock_i8(reinterpret_cast<const uint8_t *>(idx->d_stage_buf[cur]), r0 - row0, arena,
+                                          dst0 + (r0 - lo), r1 - r0, s);
+                return e;
+            });
+        }
+        dst += cnt;
     }
-    fclose(f);
-    cudaError_t se = cudaStreamSynchronize(idx->stream);
-    idx->stage_busy[0] = idx->stage_busy[1] = false;
+    if (ok && ce == cudaSuccess && n && idx->scalar == DAWN_SCALAR_F32)
+        ce = launch_ingest_f16(f->corpus32, nc, (size_t)n, s, true);  // rebuild the selection copy
+    const cudaError_t se = cudaStreamSynchronize(s);
     if (ce == cudaSuccess) ce = se;
-    if (!ok || ce != cudaSuccess) {
-        if (!in_place) {
-            cudaFree(nc);
-            cudaFree(nl);
-            cudaFree(n32);
-        }
-        if (ce != cudaSuccess) {
-            cudaGetLastError();
-            return fail(DAWN_ERR_IO, "copy to the device failed while loading %s: %s (index unchanged)", path, cudaGetErrorString(ce));
-        }
-        return fail(DAWN_ERR_IO, "read error on %s (index unchanged)", path);
+    if (ok && ce == cudaSuccess) return DAWN_OK;
+    fill_discard(idx, f);
+    if (ce != cudaSuccess) {
+        cudaGetLastError();
+        return fail(DAWN_ERR_IO, "copy to the device failed while loading %s: %s (index unchanged)", path, cudaGetErrorString(ce));
     }
-    if (in_place) {
-        idx->size = (size_t)h.size;
-        if (idx->capacity < (size_t)h.size) idx->capacity = (size_t)h.size;
+    return fail(DAWN_ERR_IO, "read error on %s (index unchanged)", path);
+}
+
+void fill_discard(dawn_index *idx, Fill *f) {
+    if (!f->in_place && f->corpus) {
+        cudaSetDevice(idx->device);
+        cudaFree(f->corpus);
+        cudaFree(f->labels);
+        cudaFree(f->corpus32);
+    }
+    *f = Fill{};
+}
+
+void fill_commit(dawn_index *idx, Fill *f) {
+    cudaSetDevice(idx->device);
+    const size_t n = (size_t)f->rows;
+    if (f->in_place) {
+        idx->size = n;
+        if (idx->capacity < n) idx->capacity = n;
         reset_norm_stats(idx);
-        return DAWN_OK;
+        *f = Fill{};
+        return;
     }
     __half *oc;
     uint64_t *ol;
@@ -1952,20 +2078,24 @@ int dawn_index_load(dawn_index *idx, const char *path) {
         oc = idx->corpus;
         ol = idx->labels;
         o32 = idx->corpus32;
-        idx->corpus = nc;
-        idx->labels = nl;
-        idx->corpus32 = n32;
-        idx->phys = rows_alloc;
+        idx->corpus = static_cast<__half *>(f->corpus);
+        idx->labels = f->labels;
+        idx->corpus32 = f->corpus32;
+        idx->phys = f->rows_alloc;
         drop_shadow(idx);
-        idx->size = (size_t)h.size;
-        if (idx->capacity < (size_t)h.size) idx->capacity = (size_t)h.size;
+        idx->size = n;
+        if (idx->capacity < n) idx->capacity = n;
     }
     cudaFree(oc);
     cudaFree(ol);
     cudaFree(o32);
     reset_norm_stats(idx);
-    return DAWN_OK;
+    *f = Fill{};
 }
+
+}  // namespace dawn
+
+extern "C" {
 
 // ---- evidence for the certificate's constants (tests/test_gpu_slack.py) -----------------------------------
 // Every (query,row) score the tensor cores produce for `batch` host queries against an index of <= 2048 rows is compared

@@ -30,9 +30,13 @@
 
 #include <cuda_runtime.h>
 #include <dlfcn.h>
+#include <fcntl.h>
 #include <nccl.h>  // types and prototypes only: the library is bound at run time, see NcclApi
+#include <sys/stat.h>
+#include <unistd.h>
 
 #include "../../include/dawn_index.h"
+#include "persist.cuh"
 
 namespace {
 
@@ -124,6 +128,10 @@ size_t block_bytes(size_t batch, size_t k) { return (batch * k * 12 + batch * 4 
 
 struct dawn_multi {
     std::vector<Shard *> shards;
+    // Every call takes `mu` except save; the calls that change what the shards hold (save, load, add*, remove, reserve,
+    // set_option) first take `writer_mu`.  So a save, which holds writer_mu alone, keeps the shards still while it writes
+    // them out, and searches and gets go on meanwhile.
+    std::mutex writer_mu;
     std::mutex mu;
     uint32_t scalar = DAWN_SCALAR_F16;
     // device 0 side
@@ -191,6 +199,30 @@ int run_all(dawn_multi *m, const std::function<int(Shard *, size_t)> &fn) {
 int cuda_fail(cudaError_t e, const char *what) {
     g_multi_err = std::string(what) + ": " + cudaGetErrorString(e);
     return DAWN_ERR_CUDA;
+}
+
+// fn for every shard at once, each on a thread of its own, for the calls that run without mu (save, and the fill of a
+// load): the shard workers serve one caller at a time, the one holding mu, so those calls must not queue on them.
+int run_parallel(dawn_multi *m, const std::function<int(Shard *, size_t)> &fn) {
+    const size_t G = m->shards.size();
+    std::vector<int> rcs(G, DAWN_OK);
+    std::vector<std::string> errs(G);
+    std::vector<std::thread> threads;
+    for (size_t g = 0; g < G; g++)
+        threads.emplace_back([&, g] {
+            Shard *s = m->shards[g];
+            g_multi_err.clear();
+            cudaError_t e = cudaSetDevice(s->device);
+            rcs[g] = e != cudaSuccess ? cuda_fail(e, "cudaSetDevice") : fn(s, g);
+            if (rcs[g]) errs[g] = g_multi_err.empty() ? std::string(dawn_last_error()) : g_multi_err;
+        });
+    for (std::thread &t : threads) t.join();
+    for (size_t g = 0; g < G; g++)
+        if (rcs[g]) {
+            g_multi_err = errs[g];
+            return rcs[g];
+        }
+    return DAWN_OK;
 }
 
 }  // namespace
@@ -317,6 +349,7 @@ size_t dawn_multi_capacity(const dawn_multi *m) {
 // Capacity is split evenly over the shards.
 int dawn_multi_reserve(dawn_multi *m, size_t n_total) {
     if (!m) return DAWN_ERR_INVALID;
+    std::lock_guard<std::mutex> wk(m->writer_mu);
     std::lock_guard<std::mutex> lk(m->mu);
     const size_t per = (n_total + m->shards.size() - 1) / m->shards.size();
     for (Shard *s : m->shards) {
@@ -333,6 +366,7 @@ int dawn_multi_reserve(dawn_multi *m, size_t n_total) {
 // vectors, so any placement gives the same answers).
 int dawn_multi_add_batch(dawn_multi *m, const uint64_t *labels, const float *vectors, size_t n) {
     if (!m || (n && (!labels || !vectors))) return DAWN_ERR_INVALID;
+    std::lock_guard<std::mutex> wk(m->writer_mu);
     std::lock_guard<std::mutex> lk(m->mu);
     const size_t kBlock = 4096;
     size_t done = 0;
@@ -371,6 +405,7 @@ int dawn_multi_add(dawn_multi *m, uint64_t label, const float *vector384) {
 // Synthetic corpus rows [first_row, first_row+n) split into contiguous id ranges, one per shard.
 int dawn_multi_add_synthetic(dawn_multi *m, uint64_t seed, uint64_t first_row, size_t n) {
     if (!m) return DAWN_ERR_INVALID;
+    std::lock_guard<std::mutex> wk(m->writer_mu);
     std::lock_guard<std::mutex> lk(m->mu);
     const size_t G = m->shards.size();
     const size_t per = (n + G - 1) / G;
@@ -390,6 +425,7 @@ int dawn_multi_remove_batch(dawn_multi *m, const uint64_t *labels, size_t n, siz
         return DAWN_ERR_INVALID;
     }
     if (n == 0) return DAWN_OK;
+    std::lock_guard<std::mutex> wk(m->writer_mu);
     std::lock_guard<std::mutex> lk(m->mu);
     std::vector<size_t> removed(m->shards.size(), 0);
     size_t *counts = removed.data();
@@ -583,6 +619,7 @@ int dawn_multi_search_batch_limit(dawn_multi *m, const float *queries, size_t ba
 // "exchange": 0 = auto (NCCL all-gather when communicators exist), 1 = peer copies, 2 = NCCL or fail.
 int dawn_multi_set_option(dawn_multi *m, const char *key, int64_t value) {
     if (!m || !key) return DAWN_ERR_INVALID;
+    std::lock_guard<std::mutex> wk(m->writer_mu);
     std::lock_guard<std::mutex> lk(m->mu);
     if (!strcmp(key, "exchange")) {
         if (value < 0 || value > 2) return DAWN_ERR_INVALID;
@@ -632,6 +669,304 @@ int dawn_multi_search_limit(dawn_multi *m, const float *query384, size_t k, floa
 int dawn_multi_search(dawn_multi *m, const float *query384, size_t k, uint64_t *labels_out, float *distances_out,
                       size_t *count_out) {
     return dawn_multi_search_batch(m, query384, 1, k, labels_out, distances_out, count_out);
+}
+
+// ---- persistence: one file for the whole handle (include/dawn_index.h, DESIGN.md section 6) ----------------------------
+
+}  // extern "C"
+
+namespace {
+
+using dawn::SectionRef;
+
+constexpr uint64_t kMultiHeaderBytes = 4096;  // also the alignment of every section: concurrent writers never share a page
+constexpr size_t kMaxShardRows = 0xFFFFFFF0ull;  // a shard holds fewer rows than this (grow_physical's limit)
+constexpr uint64_t kMaxFileRows = 1ull << 40;    // row counts beyond this cannot come from a real file
+
+struct MultiHeader {  // the first 32 bytes of a DAWNMULT file; uint64 rows[G] follow, then zeros up to kMultiHeaderBytes
+    char magic[8];    // "DAWNMULT"
+    uint32_t version, scalar, dims, shards;
+    uint64_t next_shard;
+};
+static_assert(sizeof(MultiHeader) == 32, "file layout");
+
+// Sets off[g] to section g's start; returns the file length (the end of the last section).
+uint64_t multi_layout(uint32_t scalar, const std::vector<uint64_t> &rows, std::vector<uint64_t> &off) {
+    uint64_t end = kMultiHeaderBytes;
+    off.resize(rows.size());
+    for (size_t g = 0; g < rows.size(); g++) {
+        off[g] = (end + kMultiHeaderBytes - 1) / kMultiHeaderBytes * kMultiHeaderBytes;
+        end = off[g] + rows[g] * sizeof(uint64_t) + dawn::section_payload_bytes(scalar, rows[g]);
+    }
+    return end;
+}
+
+// The sections of a DAWNMULT file, or of a DAWNB200 single-index file (one section, cursor 0).  Everything is checked
+// against the handle's storage type and against the file's length before any device work.
+bool read_sections(int fd, uint32_t scalar, std::vector<SectionRef> *secs, uint64_t *cursor, std::string *why) {
+    unsigned char head[32];
+    struct stat st;
+    if (fstat(fd, &st) != 0 || !dawn::pread_all(fd, head, sizeof head, 0)) {
+        *why = "shorter than a header";
+        return false;
+    }
+    uint32_t version, file_scalar, dims;
+    memcpy(&version, head + 8, 4);
+    memcpy(&file_scalar, head + 12, 4);
+    memcpy(&dims, head + 16, 4);
+    uint64_t want = 0;
+    if (!memcmp(head, "DAWNB200", 8) || !memcmp(head, "DAWNMULT", 8)) {
+        if (version != 1 || file_scalar != scalar || dims != DAWN_DIMENSIONS) {
+            *why = "version, storage type or dimensions differ from this handle's";
+            return false;
+        }
+    } else {
+        *why = "not a libdawn_b200 index file";
+        return false;
+    }
+    if (!memcmp(head, "DAWNB200", 8)) {
+        uint64_t size;
+        memcpy(&size, head + 24, 8);
+        if (size > kMaxFileRows) {
+            *why = "row count out of range";
+            return false;
+        }
+        secs->assign(1, SectionRef{sizeof head, size});
+        *cursor = 0;
+        want = sizeof head + size * sizeof(uint64_t) + dawn::section_payload_bytes(scalar, size);
+    } else {
+        MultiHeader h;
+        memcpy(&h, head, sizeof h);
+        if (h.shards < 1 || h.shards > 64 || h.next_shard >= h.shards) {
+            *why = "shard count or add cursor out of range";
+            return false;
+        }
+        std::vector<uint64_t> rows(h.shards), off;
+        if (!dawn::pread_all(fd, rows.data(), rows.size() * sizeof(uint64_t), sizeof h)) {
+            *why = "header cut short";
+            return false;
+        }
+        for (uint64_t r : rows)
+            if (r > kMaxFileRows) {
+                *why = "row count out of range";
+                return false;
+            }
+        want = multi_layout(scalar, rows, off);
+        secs->clear();
+        for (size_t g = 0; g < rows.size(); g++) secs->push_back(SectionRef{off[g], rows[g]});
+        *cursor = h.next_shard;
+    }
+    if ((uint64_t)st.st_size != want) {
+        *why = "file length " + std::to_string((long long)st.st_size) + " differs from the " + std::to_string(want) +
+               " bytes its header implies";
+        return false;
+    }
+    return true;
+}
+
+int io_fail(const char *path, const std::string &why) {
+    g_multi_err = std::string(path) + ": " + why;
+    return DAWN_ERR_IO;
+}
+
+}  // namespace
+
+extern "C" {
+
+// Header, then each shard's section written by a thread of its own (pwrite at its own page-aligned offset), to path.tmp,
+// renamed when every section is on disk.  Holds only writer_mu: adds and removes wait, searches and gets go on.
+int dawn_multi_save(dawn_multi *m, const char *path) {
+    if (!m || !path) {
+        g_multi_err = !m ? "null multi handle" : "path is null";
+        return DAWN_ERR_INVALID;
+    }
+    std::lock_guard<std::mutex> wk(m->writer_mu);
+    const size_t G = m->shards.size();
+    std::vector<uint64_t> rows(G), off;
+    uint64_t *r = rows.data();
+    int rc = run_parallel(m, [=](Shard *s, size_t g) -> int { return dawn::section_prepare(s->idx, false, r + g); });
+    if (rc) return rc;
+    const uint64_t len = multi_layout(m->scalar, rows, off);
+    std::vector<unsigned char> head(kMultiHeaderBytes, 0);
+    MultiHeader h{};
+    memcpy(h.magic, "DAWNMULT", 8);
+    h.version = 1;
+    h.scalar = m->scalar;
+    h.dims = DAWN_DIMENSIONS;
+    h.shards = (uint32_t)G;
+    h.next_shard = m->next_shard % G;
+    memcpy(head.data(), &h, sizeof h);
+    memcpy(head.data() + sizeof h, rows.data(), G * sizeof(uint64_t));
+    const std::string tmp = std::string(path) + ".tmp";
+    const int fd = open(tmp.c_str(), O_WRONLY | O_CREAT | O_TRUNC | O_CLOEXEC, 0666);
+    if (fd < 0) return io_fail(tmp.c_str(), "cannot open for writing");
+    // the gaps between sections are holes of the right length, read back as the zero padding
+    if (ftruncate(fd, (off_t)len) != 0 || !dawn::pwrite_all(fd, head.data(), head.size(), 0)) {
+        rc = io_fail(tmp.c_str(), "short write");
+    } else {
+        const uint64_t *o = off.data();
+        rc = run_parallel(m, [=](Shard *s, size_t g) -> int { return dawn::section_write(s->idx, fd, o[g], r[g]); });
+    }
+    const int frc = dawn::finish_file(fd, tmp.c_str(), path, rc);
+    if (frc != rc) g_multi_err = dawn_last_error();
+    return frc;
+}
+
+// Phase 1 fills every shard at once (run_parallel); phase 2 publishes all of them under mu, so no search sees old and new shards
+// mixed, and a failure of any shard leaves the handle as it was.  Same shard count: section g -> shard g and the add cursor
+// is restored.  Otherwise the sections are concatenated and shard g gets rows [g P, min(N, (g+1) P)), P = ceil(N / G),
+// cursor 0.
+int dawn_multi_load(dawn_multi *m, const char *path) {
+    if (!m || !path) {
+        g_multi_err = !m ? "null multi handle" : "path is null";
+        return DAWN_ERR_INVALID;
+    }
+    std::lock_guard<std::mutex> wk(m->writer_mu);
+    const size_t G = m->shards.size();
+    const int fd = open(path, O_RDONLY | O_CLOEXEC);
+    if (fd < 0) return io_fail(path, "cannot open");
+    std::vector<SectionRef> secs;
+    uint64_t cursor = 0;
+    std::string why;
+    if (!read_sections(fd, m->scalar, &secs, &cursor, &why)) {
+        close(fd);
+        return io_fail(path, why);
+    }
+    uint64_t total = 0;
+    for (const SectionRef &sr : secs) total += sr.rows;
+    std::vector<uint64_t> first(G), count(G);
+    const uint64_t per = (total + G - 1) / G;
+    for (size_t g = 0, at = 0; g < G; g++) {
+        if (secs.size() == G) {
+            first[g] = at;
+            count[g] = secs[g].rows;
+            at += secs[g].rows;
+        } else {
+            first[g] = g * per < total ? g * per : total;
+            count[g] = first[g] + per < total ? per : total - first[g];
+        }
+        if (count[g] >= kMaxShardRows) {
+            close(fd);
+            return io_fail(path, "more rows per shard than one GPU's index holds");
+        }
+    }
+    if (secs.size() != G) cursor = 0;
+    const bool was_empty = dawn_multi_size(m) == 0;
+    std::vector<dawn::Fill> fills(G);
+    dawn::Fill *fp = fills.data();
+    const SectionRef *sp = secs.data();
+    const size_t n_secs = secs.size();
+    const uint64_t *fi = first.data(), *co = count.data();
+    int rc = run_parallel(m, [=](Shard *s, size_t g) -> int {
+        uint64_t held = 0;
+        int r = dawn::section_prepare(s->idx, false, &held);  // flushes staged adds: they belong to the old contents
+        if (r) return r;
+        return dawn::fill_rows(s->idx, fd, path, sp, n_secs, fi[g], co[g], was_empty, fp + g);
+    });
+    close(fd);
+    if (rc) {
+        for (size_t g = 0; g < G; g++) dawn::fill_discard(m->shards[g]->idx, &fills[g]);
+        return rc;
+    }
+    std::lock_guard<std::mutex> lk(m->mu);
+    for (size_t g = 0; g < G; g++) dawn::fill_commit(m->shards[g]->idx, &fills[g]);
+    m->next_shard = cursor;
+    return DAWN_OK;
+}
+
+// Every shard looks the label up at once; the lowest-index shard holding it answers (the copy the merge keeps).
+int dawn_multi_get(dawn_multi *m, uint64_t label, float *out384) {
+    if (!m || !out384) {
+        g_multi_err = !m ? "null multi handle" : "output is null";
+        return DAWN_ERR_INVALID;
+    }
+    std::lock_guard<std::mutex> lk(m->mu);
+    const size_t G = m->shards.size();
+    std::vector<float> vec(G * DAWN_DIMENSIONS);
+    std::vector<int> rcs(G, DAWN_OK);
+    std::vector<std::string> errs(G);
+    float *v = vec.data();
+    int *rp = rcs.data();
+    std::string *ep = errs.data();
+    run_all(m, [=](Shard *s, size_t g) -> int {
+        rp[g] = dawn_index_get(s->idx, label, v + g * DAWN_DIMENSIONS);
+        if (rp[g]) ep[g] = dawn_last_error();
+        return DAWN_OK;
+    });
+    for (size_t g = 0; g < G; g++)
+        if (rcs[g] != DAWN_OK && rcs[g] != DAWN_ERR_INVALID) {  // a CUDA error, not an absent label
+            g_multi_err = errs[g];
+            return rcs[g];
+        }
+    for (size_t g = 0; g < G; g++)
+        if (rcs[g] == DAWN_OK) {
+            memcpy(out384, v + g * DAWN_DIMENSIONS, DAWN_DIMENSIONS * sizeof(float));
+            return DAWN_OK;
+        }
+    g_multi_err = "label " + std::to_string((unsigned long long)label) + " not found";
+    return DAWN_ERR_INVALID;
+}
+
+int dawn_multi_get_i24(dawn_multi *m, uint64_t label, uint8_t *out1152) {
+    if (!out1152) {
+        g_multi_err = "output is null";
+        return DAWN_ERR_INVALID;
+    }
+    float v[DAWN_DIMENSIONS];
+    int rc = dawn_multi_get(m, label, v);
+    if (rc != DAWN_OK) return rc;
+    dawn_encode_i24(v, out1152);
+    return DAWN_OK;
+}
+
+// dawn_index_verify on every shard: bad rows summed, the smallest norm over non-empty shards (0 if all are empty), the largest.
+int dawn_multi_verify(dawn_multi *m, size_t *bad_rows_out, float *min_norm_out, float *max_norm_out) {
+    if (!m) {
+        g_multi_err = "null multi handle";
+        return DAWN_ERR_INVALID;
+    }
+    std::lock_guard<std::mutex> lk(m->mu);
+    const size_t G = m->shards.size();
+    std::vector<size_t> bad(G, 0), rows(G, 0);
+    std::vector<float> lo(G, 0.f), hi(G, 0.f);
+    size_t *bp = bad.data(), *np = rows.data();
+    float *lp = lo.data(), *hp = hi.data();
+    int rc = run_all(m, [=](Shard *s, size_t g) -> int {
+        int r = dawn_index_verify(s->idx, bp + g, lp + g, hp + g);
+        np[g] = dawn_index_size(s->idx);
+        return r;
+    });
+    if (rc) return rc;
+    size_t sum = 0;
+    float mn = 0.f, mx = 0.f;
+    bool any = false;
+    for (size_t g = 0; g < G; g++) {
+        sum += bad[g];
+        mx = hi[g] > mx ? hi[g] : mx;
+        if (rows[g]) {
+            mn = !any || lo[g] < mn ? lo[g] : mn;
+            any = true;
+        }
+    }
+    if (bad_rows_out) *bad_rows_out = sum;
+    if (min_norm_out) *min_norm_out = mn;
+    if (max_norm_out) *max_norm_out = mx;
+    return DAWN_OK;
+}
+
+// The peer side of a remote search over the whole handle: decoded as dawn_index_search_i24 does.
+int dawn_multi_search_i24(dawn_multi *m, const uint8_t *query1152, size_t k, int has_limit, float distance_limit,
+                          uint64_t *labels_out, float *distances_out, size_t *count_out) {
+    if (!m || !query1152) {
+        g_multi_err = !m ? "null multi handle" : "query is null";
+        return DAWN_ERR_INVALID;
+    }
+    float q[DAWN_DIMENSIONS];
+    if (dawn_decode_i24(query1152, q) != DAWN_OK) {
+        g_multi_err = "Embedding is not normalized";
+        return DAWN_ERR_INVALID;
+    }
+    return dawn_multi_search_limit(m, q, k, has_limit ? distance_limit : NAN, labels_out, distances_out, count_out);
 }
 
 }  // extern "C"

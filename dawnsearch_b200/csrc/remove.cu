@@ -211,19 +211,25 @@ __global__ void __launch_bounds__(256) remove_pair_kernel(const uint32_t *__rest
     }
 }
 
+// Lanes 0-23 of a warp move row `from_row` of the blocked int8 arena `from` (24 x 16 B) to row `to_row` of `to`; lane 24
+// moves its scale.
+__device__ inline void move_i8_row(const uint8_t *from, size_t from_row, uint8_t *to, size_t to_row, int lane) {
+    if (lane < 24) {
+        const uint4 v = *reinterpret_cast<const uint4 *>(from + i8_row_offset(from_row) + lane * 16);
+        *reinterpret_cast<uint4 *>(to + i8_row_offset(to_row) + lane * 16) = v;
+    } else if (lane == 24) {
+        *reinterpret_cast<float *>(to + i8_scale_offset(to_row)) = *reinterpret_cast<const float *>(from + i8_scale_offset(from_row));
+    }
+}
+
 // One warp per (hole, donor) pair.  Holes lie below the cut and donors above it, so no pair reads what another writes.
 __global__ void __launch_bounds__(256) remove_move_kernel(RemoveMove p) {
     const int lane = threadIdx.x & 31;
     const size_t n_warps = ((size_t)gridDim.x * blockDim.x) >> 5;
     for (size_t i = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < p.n_pairs; i += n_warps) {
         const size_t hole = p.holes[i], donor = p.donors[i];
-        if (p.i8) {  // DAWN_SCALAR_I8: the int8 row (24 x 16 B) and its scale in the blocked layout
-            if (lane < 24) {
-                const uint4 v = *reinterpret_cast<const uint4 *>(p.arena + i8_row_offset(donor) + lane * 16);
-                *reinterpret_cast<uint4 *>(p.arena + i8_row_offset(hole) + lane * 16) = v;
-            } else if (lane == 24) {
-                *reinterpret_cast<float *>(p.arena + i8_scale_offset(hole)) = *reinterpret_cast<const float *>(p.arena + i8_scale_offset(donor));
-            }
+        if (p.i8) {  // DAWN_SCALAR_I8: the int8 row and its scale in the blocked layout
+            move_i8_row(p.arena, donor, p.arena, hole, lane);
         } else {  // the fp16 row: 48 x 16 B
             const uint4 *src = reinterpret_cast<const uint4 *>(p.arena + donor * kRowBytesF16);
             uint4 *dst = reinterpret_cast<uint4 *>(p.arena + hole * kRowBytesF16);
@@ -236,16 +242,19 @@ __global__ void __launch_bounds__(256) remove_move_kernel(RemoveMove p) {
 #pragma unroll
             for (int j = 0; j < 3; j++) dst[lane + 32 * j] = src[lane + 32 * j];
         }
-        if (p.shadow) {  // the int8 shadow row keeps ITS OWN scale, which its kappa bound was measured with
-            if (lane < 24) {
-                const uint4 v = *reinterpret_cast<const uint4 *>(p.shadow + i8_row_offset(donor) + lane * 16);
-                *reinterpret_cast<uint4 *>(p.shadow + i8_row_offset(hole) + lane * 16) = v;
-            } else if (lane == 24) {
-                *reinterpret_cast<float *>(p.shadow + i8_scale_offset(hole)) = *reinterpret_cast<const float *>(p.shadow + i8_scale_offset(donor));
-            }
-        }
+        if (p.shadow)  // the int8 shadow row keeps ITS OWN scale, which its kappa bound was measured with
+            move_i8_row(p.shadow, donor, p.shadow, hole, lane);
         if (lane == 31) p.labels[hole] = p.labels[donor];
     }
+}
+
+// One warp per row.  src (staged source blocks) and dst are different buffers.
+__global__ void __launch_bounds__(256) reblock_i8_kernel(const uint8_t *__restrict__ src, size_t src_first, uint8_t *__restrict__ dst,
+                                                         size_t dst_first, size_t n) {
+    const int lane = threadIdx.x & 31;
+    const size_t n_warps = ((size_t)gridDim.x * blockDim.x) >> 5;
+    for (size_t i = ((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < n; i += n_warps)
+        move_i8_row(src, src_first + i, dst, dst_first + i, lane);
 }
 
 inline unsigned grid_for(size_t items, size_t per_block) {
@@ -293,6 +302,12 @@ cudaError_t launch_remove_pair(const void *scratch, size_t m, size_t n, uint32_t
 cudaError_t launch_remove_move(const RemoveMove &p, cudaStream_t s) {
     if (p.n_pairs == 0) return cudaSuccess;
     remove_move_kernel<<<grid_for(p.n_pairs, 8), 256, 0, s>>>(p);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_reblock_i8(const uint8_t *src, size_t src_first, uint8_t *dst, size_t dst_first, size_t n, cudaStream_t s) {
+    if (n == 0) return cudaSuccess;
+    reblock_i8_kernel<<<grid_for(n, 8), 256, 0, s>>>(src, src_first, dst, dst_first, n);
     return cudaGetLastError();
 }
 

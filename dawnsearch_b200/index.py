@@ -221,6 +221,12 @@ def load_library() -> C.CDLL:
     L.dawn_multi_last_error.restype = C.c_char_p
     L.dawn_multi_set_option.argtypes = [_vp, C.c_char_p, C.c_int64]
     L.dawn_multi_get_stats.argtypes = [_vp, C.POINTER(MultiStats)]
+    L.dawn_multi_save.argtypes = [_vp, C.c_char_p]
+    L.dawn_multi_load.argtypes = [_vp, C.c_char_p]
+    L.dawn_multi_get.argtypes = [_vp, C.c_uint64, _vp]
+    L.dawn_multi_get_i24.argtypes = [_vp, C.c_uint64, _vp]
+    L.dawn_multi_verify.argtypes = [_vp, _vp, _vp, _vp]
+    L.dawn_multi_search_i24.argtypes = [_vp, _vp, C.c_size_t, C.c_int, C.c_float, _vp, _vp, _vp]
     _lib = L
     return L
 
@@ -610,6 +616,41 @@ class MultiIndex:
         st = MultiStats()
         self._check(self._L.dawn_multi_get_stats(self._h, C.byref(st)))
         return st.as_dict()
+
+    def save(self, path: str) -> None:
+        """One file for the whole handle (include/dawn_index.h: dawn_multi_save); searches go on while it is written."""
+        self._check(self._L.dawn_multi_save(self._h, os.fsencode(path)))
+
+    def load(self, path: str) -> None:
+        """A dawn_multi_save file or a single-index file, onto this handle's shards, whatever their number."""
+        self._check(self._L.dawn_multi_load(self._h, os.fsencode(path)))
+
+    view = load
+
+    def get(self, label: int) -> np.ndarray:
+        out = np.zeros(EM_LEN, dtype=np.float32)
+        self._check(self._L.dawn_multi_get(self._h, int(label), _ptr(out)))
+        return out
+
+    def get_i24(self, label: int) -> bytes:
+        out = np.zeros(EM_LEN * 3, dtype=np.uint8)
+        self._check(self._L.dawn_multi_get_i24(self._h, int(label), _ptr(out)))
+        return out.tobytes()
+
+    def verify(self) -> dict:
+        bad = C.c_size_t(0)
+        lo, hi = C.c_float(0), C.c_float(0)
+        self._check(self._L.dawn_multi_verify(self._h, C.byref(bad), C.byref(lo), C.byref(hi)))
+        return {"bad_rows": int(bad.value), "min_norm": float(lo.value), "max_norm": float(hi.value)}
+
+    def search_i24(self, query1152: bytes, count: int, distance_limit=None) -> Matches:
+        buf = np.frombuffer(query1152, dtype=np.uint8).copy()
+        labels = np.zeros(max(count, 1), dtype=np.uint64)
+        dist = np.zeros(max(count, 1), dtype=np.float32)
+        n = C.c_size_t(0)
+        self._check(self._L.dawn_multi_search_i24(self._h, _ptr(buf), count, int(distance_limit is not None),
+                                                  float(distance_limit or 0.0), _ptr(labels), _ptr(dist), C.byref(n)))
+        return Matches(labels[: n.value].copy(), dist[: n.value].copy())
 
 
 def new_index(options: IndexOptions | None = None) -> Index:

@@ -269,6 +269,34 @@ typedef struct dawn_multi_stats {
     uint32_t nccl_ready, reserved_;
 } dawn_multi_stats;
 int dawn_multi_get_stats(dawn_multi *m, dawn_multi_stats *out);
+/* Persistence of the whole handle (DESIGN.md section 6).  dawn_multi_save writes ONE file, little-endian:
+ *   0 "DAWNMULT", 8 u32 version = 1, 12 u32 scalar (DAWN_SCALAR_*), 16 u32 dims = 384, 20 u32 G (shards, 1..64),
+ *   24 u64 add cursor (< G), 32 u64 rows[G], zeros up to byte 4096; then one section per shard, section 0 at 4096 and
+ *   section g at the end of section g-1 rounded up to a multiple of 4096 (zero padding).  A section is u64 labels[rows],
+ *   then the stored rows exactly as dawn_index_save writes them after its header.  The file ends with the last section.
+ * Every shard writes its own section concurrently, to path.tmp, renamed when all are written; a failure removes the
+ * temporary file and leaves path alone.  A save holds adds, removes, reserve, load and set_option off, never searches or
+ * get.  Saving twice gives the same bytes, and so does save -> load (same shard count) -> save.
+ * dawn_multi_load reads a DAWNMULT file or a dawn_index_save file (one section, cursor 0) into a handle with any number
+ * of shards.  Same shard count: section g goes to shard g and the add cursor is restored.  Otherwise the N rows of all
+ * sections, in order, are split as dawn_multi_add_synthetic splits: shard g gets rows [g P, min(N, (g+1) P)),
+ * P = ceil(N / shards), cursor 0.  Stored rows are copied, never re-quantised.  Header, storage type, dimensions, shard
+ * count, cursor, file length and rows per shard are checked first (DAWN_ERR_IO); the load fills every shard, then
+ * publishes all of them at once, so a failure leaves the handle exactly as it was and no search sees a mix.  An empty
+ * handle whose shards were reserved for their share is filled in place.  With every label stored once, answers do not
+ * depend on placement; a label stored several times may come back differently after a load into another shard count,
+ * as after any add (see dawn_merge_results_device). */
+int dawn_multi_save(dawn_multi *m, const char *path);
+int dawn_multi_load(dawn_multi *m, const char *path);
+/* dawn_index_get on every shard: the lowest-index shard holding the label answers with its lowest row (the copy the merge
+ * keeps).  DAWN_ERR_INVALID if no shard holds it; a CUDA error on any shard is returned as such. */
+int dawn_multi_get(dawn_multi *m, uint64_t label, float *out384);
+int dawn_multi_get_i24(dawn_multi *m, uint64_t label, uint8_t *out1152);
+/* dawn_index_verify on every shard: bad_rows summed, min_norm over non-empty shards (0 if all are empty), max_norm the largest. */
+int dawn_multi_verify(dawn_multi *m, size_t *bad_rows_out, float *min_norm_out, float *max_norm_out);
+/* dawn_index_search_i24 over the handle: DAWN_ERR_INVALID when the decoded query is not normalised, else dawn_multi_search_limit. */
+int dawn_multi_search_i24(dawn_multi *m, const uint8_t *query1152, size_t k, int has_limit, float distance_limit,
+                          uint64_t *labels_out, float *distances_out, size_t *count_out);
 
 /* ---- instrumentation ------------------------------------------------------------------- */
 typedef struct dawn_profile {

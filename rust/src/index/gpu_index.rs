@@ -54,6 +54,12 @@ extern "C" {
     fn dawn_multi_capacity(m: *const c_void) -> usize;
     fn dawn_multi_shards(m: *const c_void) -> usize;
     fn dawn_multi_last_error() -> *const c_char;
+    fn dawn_multi_save(m: *mut c_void, path: *const c_char) -> c_int;
+    fn dawn_multi_load(m: *mut c_void, path: *const c_char) -> c_int;
+    fn dawn_multi_get(m: *mut c_void, label: u64, out384: *mut f32) -> c_int;
+    fn dawn_multi_get_i24(m: *mut c_void, label: u64, out1152: *mut u8) -> c_int;
+    fn dawn_multi_verify(m: *mut c_void, bad_rows: *mut usize, min_norm: *mut f32, max_norm: *mut f32) -> c_int;
+    fn dawn_multi_search_i24(m: *mut c_void, q1152: *const u8, k: usize, has_limit: c_int, distance_limit: f32, labels: *mut u64, dist: *mut f32, count: *mut usize) -> c_int;
 }
 
 #[derive(Clone, Copy)] pub enum MetricKind { IP }
@@ -191,6 +197,7 @@ impl Drop for Index { fn drop(&mut self) { unsafe { dawn_index_free(self.h) } } 
 /// on-box analogue of `search_remote` (src/search/search_service.rs:201-277).
 pub struct MultiIndex { m: *mut c_void }
 unsafe impl Send for MultiIndex {}
+unsafe impl Sync for MultiIndex {}  // every call serialises inside the library as Index's do; a save lets searches and get go on
 fn merr() -> anyhow::Error {
     anyhow::anyhow!(unsafe { CStr::from_ptr(dawn_multi_last_error()) }.to_string_lossy().into_owned())
 }
@@ -251,6 +258,38 @@ impl MultiIndex {
     pub fn size(&self) -> usize { unsafe { dawn_multi_size(self.m) } }
     pub fn capacity(&self) -> usize { unsafe { dawn_multi_capacity(self.m) } }
     pub fn shards(&self) -> usize { unsafe { dawn_multi_shards(self.m) } }
+    /// One file for the whole index (every shard writes its section at once); searches go on while it is written.  :117,178
+    pub fn save(&self, path: &str) -> anyhow::Result<()> { let p = CString::new(path)?; mck(unsafe { dawn_multi_save(self.m, p.as_ptr()) }) }
+    /// A `save` file or a single-GPU `Index::save` file, onto however many GPUs this handle has; all or nothing.  :115
+    pub fn load(&self, path: &str) -> anyhow::Result<()> { let p = CString::new(path)?; mck(unsafe { dawn_multi_load(self.m, p.as_ptr()) }) }
+    pub fn view(&self, path: &str) -> anyhow::Result<()> { self.load(path) }
+    /// `embedding_for_page` (search_provider.rs:183-195): the copy on the lowest-index shard holding the label.
+    pub fn get(&self, label: u64) -> anyhow::Result<Vec<f32>> {
+        let mut v = vec![0f32; 384];
+        mck(unsafe { dawn_multi_get(self.m, label, v.as_mut_ptr()) })?;
+        Ok(v)
+    }
+    /// `GetEmbedding` over UDP (udp_service.rs:254-276).
+    pub fn get_i24(&self, label: u64) -> anyhow::Result<Vec<u8>> {
+        let mut v = vec![0u8; 1152];
+        mck(unsafe { dawn_multi_get_i24(self.m, label, v.as_mut_ptr()) })?;
+        Ok(v)
+    }
+    /// `SearchProvider::verify` (search_provider.rs:289-327) over every shard: (bad rows summed, min |v|, max |v|).
+    pub fn verify(&self) -> anyhow::Result<(usize, f32, f32)> {
+        let (mut bad, mut lo, mut hi) = (0usize, 0f32, 0f32);
+        mck(unsafe { dawn_multi_verify(self.m, &mut bad, &mut lo, &mut hi) })?;
+        Ok((bad, lo, hi))
+    }
+    /// The peer side of a remote search (udp_service.rs:174-213): the 1152-byte i24 embedding straight off the wire.
+    pub fn search_i24(&self, wire: &[u8], count: usize, distance_limit: Option<f32>) -> anyhow::Result<Matches> {
+        anyhow::ensure!(wire.len() == 1152, "i24 embedding must be 1152 bytes");
+        let (mut labels, mut distances, mut n) = (vec![0u64; count], vec![0f32; count], 0usize);
+        mck(unsafe { dawn_multi_search_i24(self.m, wire.as_ptr(), count, distance_limit.is_some() as c_int, distance_limit.unwrap_or(0.0),
+                                           labels.as_mut_ptr(), distances.as_mut_ptr(), &mut n) })?;
+        labels.truncate(n); distances.truncate(n);
+        Ok(Matches { labels, distances })
+    }
 }
 impl Drop for MultiIndex { fn drop(&mut self) { unsafe { dawn_multi_free(self.m) } } }
 
